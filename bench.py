@@ -16,6 +16,7 @@ The ONE JSON line of the default run also carries, as extra keys (each its own m
   single_clip            BASELINE config 1: one 4 s clip, batch 1, eager and as a CUDA graph          (N = 1)
   longform               BASELINE config 4: a 10-minute clip, windows sharded over the N ranks
 `--workload train|single|longform` print one of these as its own line instead.
+`--dump-outputs DIR` writes the waves the last timed step of the headline workload returned (see dump_outputs).
 """
 import argparse
 import json
@@ -26,6 +27,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "unet-phasegen_b200")):
     if p not in sys.path:
@@ -42,6 +44,7 @@ CLIPS_PER_GPU = 256
 DEFAULT_PRECISION = "f16mix1"
 METRIC = "audio_seconds_per_second_mag_to_phase_to_wave"
 UNIT = "audio-s/s"
+DUMP_BYTES = 64 * 2 ** 20
 
 
 def workload_geometry():
@@ -49,6 +52,20 @@ def workload_geometry():
     T = synth.frames_for(SECONDS, SR, HOP)
     N = (T - 1) * HOP
     return T, N, N / SR
+
+
+def dump_outputs(out_dir, audio):
+    """Write the waves [B, N] one headline step returned, so that two builds can be compared output for output on the
+    same seeded inputs: out_dir/audio.npy (float32 [k, N]) holds k evenly spaced clips of the batch (all of them when they
+    fit), as many as keep the dump under DUMP_BYTES, and out_dir/audio_clips.npy (float64 [k]) their indices in the batch."""
+    import numpy as np
+    import torch
+    B, N = audio.shape
+    k = max(1, min(B, (DUMP_BYTES - 2 ** 20) // (4 * N)))
+    idx = np.unique(np.linspace(0, B - 1, k).round().astype(np.int64))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "audio.npy"), audio[torch.from_numpy(idx).to(audio.device)].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "audio_clips.npy"), idx.astype(np.float64))
 
 
 def unet_flops_per_clip(C, T, phase_only):
@@ -464,8 +481,7 @@ def longform_leg(args, D, net):
         out[0] = longform.process_long(pipe, wave, frames=T, batch=CLIPS_PER_GPU + 64)
     for _ in range(2):
         run()
-    steps = max(3, args.steps)
-    ms = D.timed(run, steps) / steps
+    ms = D.timed(run, args.steps) / args.steps
     y = out[0]
     finite = bool(torch.isfinite(y).all())
     peak = float(y.abs().max())
@@ -547,7 +563,12 @@ def main():
     ap.add_argument("--train-c", type=int, default=1024)
     ap.add_argument("--train-fp32", action="store_true", help="train with the fp32-class bf16x3 products instead of bf16")
     ap.add_argument("--longform-minutes", type=float, default=10.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step of the headline workload returned (rank 0) "
+                         "as .npy files under DIR: the waves of evenly spaced clips, at most 64 MB")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "phasegen" or args.workload != "infer"):
+        ap.error("--dump-outputs applies to the headline workload (--impl phasegen --workload infer)")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -586,9 +607,10 @@ def main():
     host_in = synth.synthetic_waves(B, N, SR, seed=100 + rank).pin_memory()
     host_out = torch.empty(B, N, dtype=torch.float32).pin_memory()
     wave = host_in.to(dev)
+    last = [None]
 
     def step_resident():
-        return pipe(wave)
+        last[0] = pipe(wave)
 
     def step_e2e_sync():
         # the public host-buffer call, one batch at a time: pinned host wave in, pinned host wave out, copies inside;
@@ -626,6 +648,8 @@ def main():
     ms = D.timed(step_resident, args.steps)
     launches = _lib.launches - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last[0])
     for _ in range(2):
         step_e2e_sync()
     ms_e2e_sync = D.timed(step_e2e_sync, args.steps)

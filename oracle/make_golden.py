@@ -1,14 +1,16 @@
 """Generate tests/golden/*.npz by RUNNING THE UNMODIFIED REFERENCE.  Build-container only.
 
-    python oracle/make_golden.py            # needs /root/reference (absent on the GPU box)
+    python oracle/make_golden.py REF_DIR    # REF_DIR: a checkout of LemonATsu/UNet-PhaseGen
 
 What it pins:
-  * unet_c{C}_t{T}.npz -- /root/reference/model.py ``UNetModel(C, 2C, norm_layer=BatchNorm1d)``
+  * unet_c{C}_t{T}.npz -- the reference's model.py ``UNetModel(C, 2C, norm_layer=BatchNorm1d)``
     in train mode (the reference never calls .eval()), float64, on seeded input:
     the input, every state_dict entry, the batch-statistics output (train.py:42 semantics),
     the per-clip output (demo.py:33-42 batch-1 loop), and the train.py:45-61 loss with the
-    gradient of two weights.  ``matplotlib``/``librosa`` are stubbed only so that model.py:7
-    (``from utils import ...``) resolves; no reference file is copied or modified.
+    gradient of four weights (the two largest of the C=16 case as every 5th element of the
+    flattened tensor, with ``stride::<name>`` = 5, which keeps the file under 1 MB).
+    ``matplotlib``/``librosa`` are stubbed only so that model.py:7 (``from utils import ...``)
+    resolves; no reference file is copied or modified.
   * stft_*.npz -- the reference has no STFT code of its own (librosa, not installed), so
     these hold outputs of CPU ``torch.stft``/``torch.istft`` configured to librosa's
     semantics, as an independent cross-check of oracle/stft_np.py.
@@ -23,10 +25,9 @@ import torch.nn as nn
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 OUT = os.path.join(HERE, "..", "tests", "golden")
-REF = "/root/reference"
 
 
-def import_reference_model():
+def import_reference_model(ref_dir):
     for name in ("matplotlib", "matplotlib.pyplot", "librosa", "librosa.display"):
         if name not in sys.modules:
             m = types.ModuleType(name)
@@ -34,18 +35,19 @@ def import_reference_model():
             sys.modules[name] = m
     sys.modules["matplotlib"].pyplot = sys.modules["matplotlib.pyplot"]
     sys.modules["librosa"].display = sys.modules["librosa.display"]
-    sys.path.insert(0, REF)
+    ref_dir = os.path.abspath(ref_dir)
+    sys.path.insert(0, ref_dir)
     try:
         for stale in ("model", "utils"):
             sys.modules.pop(stale, None)
         import model as ref_model
     finally:
-        sys.path.remove(REF)
-    assert os.path.dirname(os.path.abspath(ref_model.__file__)) == REF
+        sys.path.remove(ref_dir)
+    assert os.path.dirname(os.path.abspath(ref_model.__file__)) == ref_dir
     return ref_model
 
 
-def unet_case(ref_model, C, T, B, seed):
+def unet_case(ref_model, C, T, B, seed, grad_stride=1):
     torch.manual_seed(seed)
     net = ref_model.UNetModel(C, 2 * C, norm_layer=nn.BatchNorm1d).double()
     net.train()
@@ -77,6 +79,10 @@ def unet_case(ref_model, C, T, B, seed):
            "grad::model.1.model.3.model.3.model.3.weight":
                grads["model.1.model.3.model.3.model.3.weight"].numpy(),
            "grad::model.1.model.2.weight": grads["model.1.model.2.weight"].numpy()}
+    if grad_stride > 1:
+        for k in ("model.0.weight", "model.3.weight"):
+            rec["grad::" + k] = rec["grad::" + k].ravel()[::grad_stride].copy()
+            rec["stride::" + k] = np.int64(grad_stride)
     for k, v in sd.items():
         rec["sd::" + k] = v.numpy()
     np.savez_compressed(os.path.join(OUT, f"unet_c{C}_t{T}.npz"), **rec)
@@ -101,10 +107,10 @@ def stft_case(n_fft, hop, n, seed):
 
 def main():
     os.makedirs(OUT, exist_ok=True)
-    ref_model = import_reference_model()
+    ref_model = import_reference_model(sys.argv[1])
     unet_case(ref_model, 8, 24, 2, seed=1)
     unet_case(ref_model, 8, 40, 3, seed=2)
-    unet_case(ref_model, 16, 64, 2, seed=3)
+    unet_case(ref_model, 16, 64, 2, seed=3, grad_stride=5)
     stft_case(512, 128, 128 * 23, seed=4)
     stft_case(1024, 256, 256 * 15, seed=5)
     stft_case(2048, 512, 512 * 7, seed=6)

@@ -19,6 +19,13 @@ def rel_l2(a, b):
     return np.linalg.norm(a - b) / np.linalg.norm(b)
 
 
+def _stored_part(z, name, full):
+    """The elements of ``full`` that the golden file keeps for gradient ``name``: all of them, or every
+    ``stride::<name>``-th element of the flattened tensor where the file stores a strided sample (keeps it under 1 MB)."""
+    key = "stride::" + name
+    return full.ravel()[::int(z[key])] if key in z.files else full
+
+
 def _train_py_loss(pred, x, phi, C):
     """train.py:45-60 verbatim in behaviour, with torch ops on the GPU (what a user's script does)."""
     lossf = torch.nn.MSELoss()
@@ -45,7 +52,7 @@ def test_backward_matches_reference_gradients(path):
     grads = {k: p.grad for k, p in net.model.named_parameters()}
     for k in z.files:
         if k.startswith("grad::"):
-            assert rel_l2(grads[k[6:]].cpu().numpy(), z[k]) < 2e-4, k
+            assert rel_l2(_stored_part(z, k[6:], grads[k[6:]].cpu().numpy()), z[k]) < 2e-4, k
     tgt = torch.stack([torch.from_numpy(z["x"]), torch.from_numpy(z["phi"])], 1)
     _, _, _, ref = unet_torch.loss_and_grads(sd, torch.from_numpy(z["x"]), tgt)
     for k, g in ref.items():

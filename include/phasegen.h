@@ -75,6 +75,31 @@ int pg_istft(const float* in_a, const float* in_b, int mode, int B, int T, int n
              const float* b_scale_shift, int b_ss_per_clip, pg_stream stream);
 int pg_peak_normalize(float* wave, const float* peak, int B, int N, pg_stream stream);
 
+/* ---------------------------------------------------------------- ragged batches
+ * Clips of different lengths in one [B][N] buffer: clip b holds its first n_b <= N samples.  Its frame count is T_b, the
+ * smallest multiple of 8 with (T_b - 1)*hop >= n_b, and it is computed as if it were alone, zero-padded to (T_b - 1)*hop
+ * samples.  Each entry below is the NULL-lengths entry above with per-clip int32 arrays in device memory [B]; every
+ * layer of the U-Net then holds clip b's valid rows L_b (the convolution length chain from T_b) and ZEROS in rows
+ * [L_b, L), which is the zero padding the next convolution of the standalone clip would read.  Table entries larger
+ * than the call's extent (N, T, L_out, L) are clamped to it, so a bad table never reaches another clip's rows.
+ *
+ * pg_stft_ragged: PG_STFT_LOGMAG only (else PG_ERR_UNSUPPORTED).  Samples >= clip_samples[b] are never read; reflect
+ *   padding at (T_b - 1)*hop; frames >= T_b = clip_frames[b] are written as 0 in every plane.
+ * pg_conv_tc_ragged: out_rows[b] = valid output rows L_b.  PG_EPI_RAW: statistics records count those rows only (a part
+ *   with none gets n = 0, which pg_bn_finalize skips); y beyond them is unspecified.  PG_EPI_ACT / NORM_ACT: the norm
+ *   uses those rows only and rows [L_b, L_out) of both destinations are written as 0.
+ * pg_bn_act_ragged: clip_rows[b] = valid rows; y is not read beyond them and rows [L_b, L) of every destination are 0.
+ * pg_istft_ragged: frames >= clip_frames[b] are not read; the window sum of squares at the clip's end is the one of
+ *   T_b frames; peak and non-finite flags cover samples [0, (T_b - 1)*hop); samples [clip_samples[b], (T-1)*hop) are
+ *   written as 0 (pg_peak_normalize keeps them 0). */
+int pg_stft_ragged(const float* wave, int B, int N, int n_fft, int hop, const float* twiddle, int mode,
+                   float* out_a, float* out_b, uint16_t* op_hi, uint16_t* op_lo, int64_t op_batch_stride,
+                   int op_fmt, const int* clip_samples, const int* clip_frames, pg_stream stream);
+int pg_istft_ragged(const float* in_a, const float* in_b, int mode, int B, int T, int n_fft, int hop,
+                    const float* twiddle, float* wave, float* peak, int* nonfinite,
+                    const float* b_scale_shift, int b_ss_per_clip, const int* clip_frames, const int* clip_samples,
+                    pg_stream stream);
+
 /* Long-form stitching (BASELINE.json config 4; the reference cuts long audio into independent slices,
  * preproc_mdb.py:66-82, and never stitches them): n_windows windows of `win` samples, one every `step` samples
  * (win/2 <= step <= win), cross-faded over the shared samples with complementary periodic-Hann ramps -> out [n_out].
@@ -163,6 +188,10 @@ int pg_conv_epilogue_supported(const pg_conv_desc* d, int mode);
 int pg_conv_tc(const pg_conv_desc* d, const uint16_t* x_hi, const uint16_t* x_lo,
                const uint16_t* w_hi, const uint16_t* w_lo, float* y, float* stats,
                const pg_conv_epilogue* epilogue /* NULL = PG_EPI_RAW */, pg_stream stream);
+/* ragged batch (see pg_stft_ragged): out_rows [B] device int32, valid output rows of each clip */
+int pg_conv_tc_ragged(const pg_conv_desc* d, const uint16_t* x_hi, const uint16_t* x_lo,
+                      const uint16_t* w_hi, const uint16_t* w_lo, float* y, float* stats,
+                      const pg_conv_epilogue* epilogue, const int* out_rows, pg_stream stream);
 int pg_conv_stat_parts(const pg_conv_desc* d);
 /* Tiling plan of pg_conv_tc for a layer, host-only: out[16] = {n_tile, n_ntiles, clips per tile, strip rows, CTA pair,
  * merged clips, MMA groups per weight tile, TMEM accumulator stages, C_in/64, C_out/128, output phases, input
@@ -193,6 +222,9 @@ int pg_bn_from_running(const float* running_mean, const float* running_var, cons
  * of leading channels of y processed. */
 int pg_bn_act(const float* y, int B, int L, int C, int rows, int ld, const float* scale_shift,
               int per_clip, const pg_act_dst* dst0, const pg_act_dst* dst1, pg_stream stream);
+/* ragged batch (see pg_stft_ragged): clip_rows [B] device int32, valid rows of each clip */
+int pg_bn_act_ragged(const float* y, int B, int L, int C, int rows, int ld, const float* scale_shift,
+                     int per_clip, const pg_act_dst* dst0, const pg_act_dst* dst1, const int* clip_rows, pg_stream stream);
 
 /* [B][R][S] fp32 -> [B][S][R] fp32 and/or 16-bit hi/lo planes (fmt = PG_FMT_*) (reference [B,C,T] <-> channels-last). */
 int pg_transpose(const float* src, int B, int R, int S, int64_t src_batch_stride, float* dst,

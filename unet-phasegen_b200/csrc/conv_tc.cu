@@ -66,6 +66,7 @@ struct ConvTcParams {
     const float* gamma; const float* beta; float eps;
     ActDst dst0, dst1;
     float2* ss_out;                 // NORM_ACT: optional [B][C_out] (scale, shift) record of what was applied
+    const int* clip_rows;           // ragged batch (RAGGED = true): valid output rows L_b <= L_out of each clip
 };
 // plan.pair = 1: tiles are 256 output channels wide and owned by a CTA pair; plan.strip_rows is then the
 // HALF strip each CTA loads (n_tile/2 + largest shift rows).
@@ -99,7 +100,10 @@ __device__ __forceinline__ TileCoord decode_tile(const ConvPlan& p, int tile) {
     return c;
 }
 
-template <bool PAIR>
+// RAGGED: clip b's output is valid in rows [0, L_b) only (prm.clip_rows).  Statistics count those rows; the fused
+// epilogues write zeros into rows [L_b, L_out) of their destinations, so a later layer reads zeros there, as TMA's
+// out-of-bounds fill supplies them to the same clip run alone.
+template <bool PAIR, bool RAGGED>
 __global__ void __launch_bounds__(kThreads, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __grid_constant__ CUtensorMap map_w_lo,
                const __grid_constant__ CUtensorMap map_x_hi, const __grid_constant__ CUtensorMap map_x_lo,
@@ -394,21 +398,23 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __grid_consta
             tc_fence_after();
             const int co_base = tc.co_tile * 128 + q * 32;
             const int co = co_base + lane;
-            // part p = (phase, position tile) of the tile: its valid columns and the output row of its column 0
-            auto part_geom = [&](int p, int& phase, int& m0, int& n_valid) {
+            // part p = (phase, position tile) of the tile: its columns among the first L output rows, and the output row
+            // of its column 0
+            auto part_geom = [&](int p, int L, int& phase, int& m0, int& n_valid) {
                 phase = tc.phase + p / t_nts;
                 m0 = (tc.nt + p % t_nts) * pl.n_tile;
-                const int l_phase = (pl.L_out - phase + pl.OS - 1) / pl.OS;   // positions of this phase
+                const int l_phase = (L - phase + pl.OS - 1) / pl.OS;          // positions of this phase
                 n_valid = l_phase - m0; if (n_valid > pl.n_tile) n_valid = pl.n_tile; if (n_valid < 0) n_valid = 0;
             };
             for (int c = 0; c < pl.nb; ++c) {
                 const int b = tc.b0 + c;
                 if (b >= pl.B) break;
+                const int L_b = RAGGED ? min(__ldg(prm.clip_rows + b), pl.L_out) : pl.L_out;   // rows holding the clip's own output
                 const uint32_t tclip = tmem_base + acc * 256 + c * col_pitch + ((uint32_t)(q * 32) << 16);
                 if (prm.epi_mode == PG_EPI_RAW) {
                     for (int p = 0; p < n_parts; ++p) {
                         int phase, m0, n_valid;
-                        part_geom(p, phase, m0, n_valid);
+                        part_geom(p, L_b, phase, m0, n_valid);
                         const uint32_t taddr = tclip + p * pl.n_tile;
                         // pass 1: mean over the valid columns
                         float sum = 0.f;
@@ -443,7 +449,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __grid_consta
                         float sum = 0.f; int n_tot = 0;
                         for (int p = 0; p < n_parts; ++p) {
                             int phase, m0, n_valid;
-                            part_geom(p, phase, m0, n_valid);
+                            part_geom(p, L_b, phase, m0, n_valid);
                             n_tot += n_valid;
                             for (int c0 = 0; c0 < n_valid; c0 += 16) {
                                 float v[16];
@@ -456,7 +462,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __grid_consta
                         float m2 = 0.f;
                         for (int p = 0; p < n_parts; ++p) {
                             int phase, m0, n_valid;
-                            part_geom(p, phase, m0, n_valid);
+                            part_geom(p, L_b, phase, m0, n_valid);
                             for (int c0 = 0; c0 < n_valid; c0 += 16) {
                                 float v[16];
                                 tmem_ld16(tclip + p * pl.n_tile + c0, v);
@@ -470,13 +476,18 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __grid_consta
                         if (prm.ss_out) prm.ss_out[(size_t)b * pl.C_out + co] = make_float2(sc, sh);
                     }
                     for (int p = 0; p < n_parts; ++p) {
-                        int phase, m0, n_valid;
-                        part_geom(p, phase, m0, n_valid);
+                        int phase, m0, n_valid, n_own = 0;
+                        part_geom(p, pl.L_out, phase, m0, n_valid);
+                        if (RAGGED) { int ph_, m0_; part_geom(p, L_b, ph_, m0_, n_own); }
                         for (int c0 = 0; c0 < n_valid; c0 += 16) {
                             float v[16];
                             tmem_ld16(tclip + p * pl.n_tile + c0, v);
 #pragma unroll
                             for (int i = 0; i < 16; ++i) v[i] = fmaf(v[i], sc, sh);
+                            if (RAGGED) {                               // rows [L_b, L_out): zeros (act(0) = 0)
+#pragma unroll
+                                for (int i = 0; i < 16; ++i) if (c0 + i >= n_own) v[i] = 0.f;
+                            }
                             const size_t row0 = (size_t)(m0 + c0) * pl.OS + phase;
 #pragma unroll
                             for (int k = 0; k < 2; ++k) {
@@ -567,8 +578,9 @@ extern "C" int pg_conv_epilogue_supported(const pg_conv_desc* d, int mode) {
     return (pl.whole_clip || (pl.OS == 1 && pl.n_ntiles == 1)) ? 1 : 0;
 }
 
-extern "C" int pg_conv_tc(const pg_conv_desc* d, const uint16_t* x_hi, const uint16_t* x_lo, const uint16_t* w_hi,
-                          const uint16_t* w_lo, float* y, float* stats, const pg_conv_epilogue* epi, pg_stream stream) {
+static int conv_tc_launch(const pg_conv_desc* d, const uint16_t* x_hi, const uint16_t* x_lo, const uint16_t* w_hi,
+                          const uint16_t* w_lo, float* y, float* stats, const pg_conv_epilogue* epi, const int* out_rows,
+                          pg_stream stream) {
     using namespace pg;
     const int epi_mode = epi ? epi->mode : PG_EPI_RAW;
     PG_REQUIRE(d && x_hi && w_hi && (y || epi_mode != PG_EPI_RAW), "pg_conv_tc: null pointer");
@@ -591,6 +603,8 @@ extern "C" int pg_conv_tc(const pg_conv_desc* d, const uint16_t* x_hi, const uin
     if (rc != PG_OK) return rc;
     const ConvPlan& pl = prm.plan;
     prm.epi_mode = epi_mode; prm.gamma = nullptr; prm.beta = nullptr; prm.eps = 1e-5f; prm.ss_out = nullptr;
+    prm.clip_rows = out_rows;
+    const bool ragged = out_rows != nullptr;
     if ((rc = to_act_dst(nullptr, 0, &prm.dst0, "pg_conv_tc", "dst0")) != PG_OK) return rc;
     prm.dst1 = prm.dst0;
     if (epi_mode != PG_EPI_RAW) {
@@ -649,14 +663,16 @@ extern "C" int pg_conv_tc(const pg_conv_desc* d, const uint16_t* x_hi, const uin
         if ((rc = encode_bf16_map(&mx_lo, n_terms >= 2 ? x_lo : x_hi, 4, dims, str, box, "x_lo")) != PG_OK) return rc;
     }
     const bool pair = pl.pair != 0;
+    auto kernel = pair ? (ragged ? conv_tc_kernel<true, true> : conv_tc_kernel<true, false>)
+                       : (ragged ? conv_tc_kernel<false, true> : conv_tc_kernel<false, false>);
     {
-        static size_t configured_dev[kMaxDevices][2] = {};
+        static size_t configured_dev[kMaxDevices][4] = {};
+        const int variant = 2 * pair + ragged;
         size_t* configured = configured_dev[current_device_slot()];
-        if (smem_bytes > configured[pair]) {
-            cudaError_t e = pair ? cudaFuncSetAttribute(conv_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes)
-                                 : cudaFuncSetAttribute(conv_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
+        if (smem_bytes > configured[variant]) {
+            cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes);
             if (e != cudaSuccess) { set_error("conv_tc: cannot opt in to %zu bytes of shared memory: %s", smem_bytes, cudaGetErrorString(e)); return PG_ERR_CUDA; }
-            configured[pair] = smem_bytes;
+            configured[variant] = smem_bytes;
         }
     }
     {
@@ -686,8 +702,19 @@ extern "C" int pg_conv_tc(const pg_conv_desc* d, const uint16_t* x_hi, const uin
     attr[0].id = cudaLaunchAttributeClusterDimension;
     attr[0].val.clusterDim.x = pair ? 2 : 1; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
-    cudaError_t le = pair ? cudaLaunchKernelEx(&cfg, conv_tc_kernel<true>, mw_hi, mw_lo, mx_hi, mx_lo, prm)
-                          : cudaLaunchKernelEx(&cfg, conv_tc_kernel<false>, mw_hi, mw_lo, mx_hi, mx_lo, prm);
+    cudaError_t le = cudaLaunchKernelEx(&cfg, kernel, mw_hi, mw_lo, mx_hi, mx_lo, prm);
     if (le != cudaSuccess) { set_error("conv_tc_kernel launch failed: %s", cudaGetErrorString(le)); return PG_ERR_CUDA; }
     return check_launch("conv_tc_kernel");
+}
+
+extern "C" int pg_conv_tc(const pg_conv_desc* d, const uint16_t* x_hi, const uint16_t* x_lo, const uint16_t* w_hi,
+                          const uint16_t* w_lo, float* y, float* stats, const pg_conv_epilogue* epi, pg_stream stream) {
+    return conv_tc_launch(d, x_hi, x_lo, w_hi, w_lo, y, stats, epi, nullptr, stream);
+}
+
+extern "C" int pg_conv_tc_ragged(const pg_conv_desc* d, const uint16_t* x_hi, const uint16_t* x_lo, const uint16_t* w_hi,
+                                 const uint16_t* w_lo, float* y, float* stats, const pg_conv_epilogue* epi, const int* out_rows,
+                                 pg_stream stream) {
+    PG_REQUIRE(out_rows, "pg_conv_tc_ragged: null per-clip row table");
+    return conv_tc_launch(d, x_hi, x_lo, w_hi, w_lo, y, stats, epi, out_rows, stream);
 }

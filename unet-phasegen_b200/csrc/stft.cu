@@ -63,13 +63,16 @@ __device__ __forceinline__ float fast_log1p_mag(float re, float im) {
 // ------------------------------------------------------------------------------------ STFT
 // FAST = 0: every output selected at run time.  FAST = 1 / 2: the inference path (log-magnitude fp32 plane +
 // bf16 / fp16 hi,lo operand planes, no phase plane) with the selection compiled in.
-template <int NC, int FAST>
+// RAGGED: clip b is its first n_b = clip_samples[b] samples zero-padded to N_b = (T_b - 1) * hop, T_b = clip_frames[b]
+// <= T: samples >= n_b are never read, reflect padding happens at N_b, and frames >= T_b are transforms of zeros, so
+// every plane holds exact zeros there.
+template <int NC, int FAST, bool RAGGED>
 __global__ void __launch_bounds__(kStftThreads, 3)          // 3 CTAs per SM (<= 85 registers): the kernel is issue/latency-bound
 stft_kernel(const float* __restrict__ wave, int N, int T, const float2* __restrict__ tw_g, int mode,
             float* __restrict__ out_a, float* __restrict__ out_b,
             uint16_t* __restrict__ op_hi, uint16_t* __restrict__ op_lo,
             long long op_batch_stride, int op_fmt, int frames_per_cta, const float* __restrict__ proj_mag,
-            float std_mean, float std_inv) {
+            float std_mean, float std_inv, const int* __restrict__ clip_samples, const int* __restrict__ clip_frames) {
     using Cfg = FrameCfg<NC>;
     using R = Radix<NC, false>;
     extern __shared__ float2 smem2[];
@@ -85,6 +88,9 @@ stft_kernel(const float* __restrict__ wave, int N, int T, const float2* __restri
     __syncthreads();
 
     const int b = blockIdx.y;
+    const int n_b = RAGGED ? min(__ldg(clip_samples + b), N) : N;   // samples read from the clip
+    const int T_b = RAGGED ? min(__ldg(clip_frames + b), T) : T;
+    const int N_b = RAGGED ? (T_b - 1) * Cfg::HOP : N;      // where the reflect padding happens
     const int slot = tid / Cfg::TG, t = tid % Cfg::TG;
     cpx* s = bufs + slot * Cfg::PL;
     const FrameSync<Cfg::TG> sync{slot};
@@ -98,7 +104,7 @@ stft_kernel(const float* __restrict__ wave, int N, int T, const float2* __restri
         // padded sample p <-> wave index p - n_fft/2, reflected at both ends (librosa center=True)
         const int p0 = frame * Cfg::HOP - NC;
         cpx v[16];
-        if (live && aligned && p0 >= 0 && p0 + Cfg::NFFT <= N) {
+        if (live && aligned && p0 >= 0 && p0 + Cfg::NFFT <= n_b) {
 #pragma unroll
             for (int r = 0; r < 16; ++r) {
                 const int m = t + r * Cfg::TG;
@@ -106,17 +112,17 @@ stft_kernel(const float* __restrict__ wave, int N, int T, const float2* __restri
                 const cpx wv = win[m];
                 v[r] = {xv.x * wv.x, xv.y * wv.y};
             }
-        } else if (live) {
+        } else if (live && (!RAGGED || frame < T_b)) {
 #pragma unroll
             for (int r = 0; r < 16; ++r) {
                 const int m = t + r * Cfg::TG;
                 int n0 = p0 + 2 * m, n1 = n0 + 1;
                 if (n0 < 0) n0 = -n0;
-                if (n0 >= N) n0 = 2 * (N - 1) - n0;
+                if (n0 >= N_b) n0 = 2 * (N_b - 1) - n0;
                 if (n1 < 0) n1 = -n1;
-                if (n1 >= N) n1 = 2 * (N - 1) - n1;
-                const float x0 = (n0 >= 0 && n0 < N) ? __ldg(w + n0) : 0.f;
-                const float x1 = (n1 >= 0 && n1 < N) ? __ldg(w + n1) : 0.f;
+                if (n1 >= N_b) n1 = 2 * (N_b - 1) - n1;
+                const float x0 = (n0 >= 0 && n0 < n_b) ? __ldg(w + n0) : 0.f;
+                const float x1 = (n1 >= 0 && n1 < n_b) ? __ldg(w + n1) : 0.f;
                 const cpx wv = win[m];
                 v[r] = {x0 * wv.x, x1 * wv.y};
             }
@@ -193,12 +199,16 @@ __device__ __forceinline__ cpx spec_value(float a, float p, int mode) {
 }
 
 // FAST: mode == PG_SPEC_POLAR_LOG with a phase plane (the inference path), selection compiled in.
-template <int NC, bool FAST>
+// RAGGED: clip b has T_b = clip_frames[b] <= T frames and n_b = clip_samples[b] <= (T_b - 1) * hop samples: frames >= T_b
+// are never read, the clip ends (window sum of squares, trim) at (T_b - 1) * hop as if it had T_b frames, peak and
+// non-finite flags cover [0, (T_b - 1) * hop), and samples [n_b, (T - 1) * hop) are written as zeros.
+template <int NC, bool FAST, bool RAGGED>
 __global__ void __launch_bounds__(kStftThreads)
 istft_kernel(const float* __restrict__ in_a, const float* __restrict__ in_b, int mode, int T,
              const float2* __restrict__ tw_g, float* __restrict__ wave,
              unsigned* __restrict__ peak_bits, int* __restrict__ nonfinite, int blocks_per_cta,
-             const float2* __restrict__ b_ss, int b_ss_stride) {
+             const float2* __restrict__ b_ss, int b_ss_stride, const int* __restrict__ clip_frames,
+             const int* __restrict__ clip_samples) {
     using Cfg = FrameCfg<NC>;
     using R = Radix<NC, true>;
     constexpr int FC = Cfg::FC, HOP = Cfg::HOP;
@@ -222,6 +232,8 @@ istft_kernel(const float* __restrict__ in_a, const float* __restrict__ in_b, int
         wss_full[i] = acc > 1.17549435e-38f ? 1.0f / acc : 1.0f;   // stored as the reciprocal: the overlap-add multiplies
     }
     const int b = blockIdx.y;
+    const int T_b = RAGGED ? min(__ldg(clip_frames + b), T) : T;   // table entries beyond the buffer are clamped to it
+    const int n_b = RAGGED ? __ldg(clip_samples + b) : 0;
     if (b_ss) for (int m = tid; m < NC; m += kStftThreads) ss_tab[m] = __ldg(b_ss + (size_t)b * b_ss_stride + m);
     __syncthreads();
 
@@ -239,7 +251,7 @@ istft_kernel(const float* __restrict__ in_a, const float* __restrict__ in_b, int
     // the 16 (a, b) input pairs of this thread's frame are fetched one iteration ahead of their use, so the
     // global-load latency hides behind the previous frame's transform and overlap-add
     float ra[16], rb[16];
-    auto is_live = [&](int frame) { return frame >= 0 && frame < T && frame <= J1 + 1; };
+    auto is_live = [&](int frame) { return frame >= 0 && frame < T_b && frame <= J1 + 1; };
     auto fetch = [&](int frame) {
         if (!is_live(frame)) return;
         const size_t row = ((size_t)b * T + frame) * NC;
@@ -279,13 +291,13 @@ istft_kernel(const float* __restrict__ in_a, const float* __restrict__ in_b, int
         for (int u = tid; u < (hi - lo) * (HOP / 4); u += kStftThreads) {
             const int jb = lo + u / (HOP / 4), i = (u % (HOP / 4)) * 4;
             float4 acc = make_float4(0.f, 0.f, 0.f, 0.f), wss;
-            const bool interior = jb >= 1 && jb + 2 < T;
+            const bool interior = jb >= 1 && jb + 2 < T_b;
             if (interior) wss = *reinterpret_cast<const float4*>(wss_full + i);   // reciprocal of the window sum of squares
             else wss = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 const int fr = jb - 1 + q;
-                if (fr < 0 || fr >= T) continue;
+                if (fr < 0 || fr >= T_b) continue;
                 const cpx* fb = ring + (size_t)((fr - F0) % Cfg::RING) * Cfg::PL;
                 const int m = ((3 - q) * HOP + i) >> 1;
                 const cpx z0 = fb[pad2(m)], z1 = fb[pad2(m + 1)];
@@ -301,10 +313,18 @@ istft_kernel(const float* __restrict__ in_a, const float* __restrict__ in_b, int
             }
             float4 y;
             y.x = acc.x * wss.x; y.y = acc.y * wss.y; y.z = acc.z * wss.z; y.w = acc.w * wss.w;
-            *reinterpret_cast<float4*>(wv + (size_t)jb * HOP + i) = y;
+            if (RAGGED && jb >= T_b - 1) y = make_float4(0.f, 0.f, 0.f, 0.f);   // past the clip's padded end
             const float mx = fmaxf(fmaxf(fabsf(y.x), fabsf(y.y)), fmaxf(fabsf(y.z), fabsf(y.w)));
             if (!(mx <= 3.402823466e+38f) || y.x != y.x || y.y != y.y || y.z != y.z || y.w != y.w) bad = true;
             pk = fmaxf(pk, mx);
+            if (RAGGED) {                                   // the zero padding of the clip is not part of its output
+                const int n = jb * HOP + i;
+                if (n >= n_b) y.x = 0.f;
+                if (n + 1 >= n_b) y.y = 0.f;
+                if (n + 2 >= n_b) y.z = 0.f;
+                if (n + 3 >= n_b) y.w = 0.f;
+            }
+            *reinterpret_cast<float4*>(wv + (size_t)jb * HOP + i) = y;
         }
         __syncthreads();                                    // the next iteration overwrites the oldest FC frames
     }
@@ -370,39 +390,49 @@ stitch_kernel(const float* __restrict__ windows, int n_windows, int win, int ste
     }
 }
 
+template <int NC, bool RAGGED>
+static auto stft_variant(bool fast, int fmt) {
+    return !fast ? stft_kernel<NC, 0, RAGGED> : fmt == PG_FMT_F16 ? stft_kernel<NC, 2, RAGGED> : stft_kernel<NC, 1, RAGGED>;
+}
+
 template <int NC>
 static int launch_stft(const float* wave, int B, int N, int T, const float* tw, int mode, float* a, float* bq,
                        uint16_t* hi, uint16_t* lo, long long bs, int fmt, cudaStream_t st, const float* proj_mag = nullptr,
-                       float std_mean = 0.f, float std_inv = 1.f) {
+                       float std_mean = 0.f, float std_inv = 1.f, const int* clip_samples = nullptr, const int* clip_frames = nullptr) {
     using Cfg = FrameCfg<NC>;
     const bool fast = mode == PG_STFT_LOGMAG && a && !bq && hi && lo;
-    auto k = !fast ? stft_kernel<NC, 0> : fmt == PG_FMT_F16 ? stft_kernel<NC, 2> : stft_kernel<NC, 1>;
+    auto k = clip_samples ? stft_variant<NC, true>(fast, fmt) : stft_variant<NC, false>(fast, fmt);
     const size_t sm = Cfg::smem_stft();
     static bool configured_dev[kMaxDevices] = {};
     bool& configured = configured_dev[current_device_slot()];
     if (!configured) {
-        cudaFuncSetAttribute(stft_kernel<NC, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        cudaFuncSetAttribute(stft_kernel<NC, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        cudaFuncSetAttribute(stft_kernel<NC, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        for (int f = 0; f < 3; ++f)
+            for (auto kv : {stft_variant<NC, false>(f > 0, f == 2 ? PG_FMT_F16 : PG_FMT_BF16),
+                            stft_variant<NC, true>(f > 0, f == 2 ? PG_FMT_F16 : PG_FMT_BF16)})
+                cudaFuncSetAttribute(kv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         configured = true;
     }
     const int frames_per_cta = Cfg::FC * 4;                 // tables are built once per 4 passes over the frame slots
     dim3 grid((T + frames_per_cta - 1) / frames_per_cta, B);
-    k<<<grid, kStftThreads, sm, st>>>(wave, N, T, reinterpret_cast<const float2*>(tw), mode, a, bq, hi, lo, bs, fmt, frames_per_cta, proj_mag, std_mean, std_inv);
+    k<<<grid, kStftThreads, sm, st>>>(wave, N, T, reinterpret_cast<const float2*>(tw), mode, a, bq, hi, lo, bs, fmt, frames_per_cta, proj_mag,
+                                      std_mean, std_inv, clip_samples, clip_frames);
     return check_launch("stft_kernel");
 }
 
 template <int NC>
 static int launch_istft(const float* a, const float* bq, int mode, int B, int T, const float* tw, float* wave,
-                        float* peak, int* nonfinite, cudaStream_t st, const float* b_ss, int b_ss_stride) {
+                        float* peak, int* nonfinite, cudaStream_t st, const float* b_ss, int b_ss_stride,
+                        const int* clip_frames = nullptr, const int* clip_samples = nullptr) {
     using Cfg = FrameCfg<NC>;
-    auto k = (mode == PG_SPEC_POLAR_LOG && bq) ? istft_kernel<NC, true> : istft_kernel<NC, false>;
+    const bool fast = mode == PG_SPEC_POLAR_LOG && bq;
+    auto k = clip_frames ? (fast ? istft_kernel<NC, true, true> : istft_kernel<NC, false, true>)
+                         : (fast ? istft_kernel<NC, true, false> : istft_kernel<NC, false, false>);
     const size_t sm = Cfg::smem_istft();
     static bool configured_dev[kMaxDevices] = {};
     bool& configured = configured_dev[current_device_slot()];
     if (!configured) {
-        cudaFuncSetAttribute(istft_kernel<NC, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
-        cudaFuncSetAttribute(istft_kernel<NC, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
+        for (auto kv : {istft_kernel<NC, true, false>, istft_kernel<NC, false, false>, istft_kernel<NC, true, true>, istft_kernel<NC, false, true>})
+            cudaFuncSetAttribute(kv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         configured = true;
     }
     // a run of 11 iterations: 11*FC - 3 output blocks per CTA, 3 halo frames recomputed per run
@@ -410,7 +440,7 @@ static int launch_istft(const float* a, const float* bq, int mode, int B, int T,
     dim3 grid((T - 1 + blocks_per_cta - 1) / blocks_per_cta, B);
     k<<<grid, kStftThreads, sm, st>>>(a, bq, mode, T, reinterpret_cast<const float2*>(tw), wave,
                                      reinterpret_cast<unsigned*>(peak), nonfinite, blocks_per_cta,
-                                     reinterpret_cast<const float2*>(b_ss), b_ss_stride);
+                                     reinterpret_cast<const float2*>(b_ss), b_ss_stride, clip_frames, clip_samples);
     return check_launch("istft_kernel");
 }
 
@@ -418,9 +448,9 @@ static int launch_istft(const float* a, const float* bq, int mode, int B, int T,
 
 extern "C" int pg_stft_num_frames(int n_samples, int hop) { return hop > 0 ? 1 + n_samples / hop : 0; }
 
-extern "C" int pg_stft(const float* wave, int B, int N, int n_fft, int hop, const float* twiddle, int mode,
-                       float* out_a, float* out_b, uint16_t* op_hi, uint16_t* op_lo,
-                       int64_t op_batch_stride, int op_fmt, pg_stream stream) {
+static int stft_entry(const float* wave, int B, int N, int n_fft, int hop, const float* twiddle, int mode,
+                      float* out_a, float* out_b, uint16_t* op_hi, uint16_t* op_lo,
+                      int64_t op_batch_stride, int op_fmt, const int* cs, const int* cf, pg_stream stream) {
     PG_REQUIRE(wave && twiddle && B > 0 && N > 0, "pg_stft: null pointer or empty batch");
     PG_REQUIRE(hop * 4 == n_fft, "pg_stft: hop must be n_fft/4 (got n_fft=%d hop=%d)", n_fft, hop);
     PG_REQUIRE(N > n_fft / 2, "pg_stft: reflect padding needs more than n_fft/2 samples (N=%d)", N);
@@ -429,13 +459,30 @@ extern "C" int pg_stft(const float* wave, int B, int N, int n_fft, int hop, cons
     const int T = 1 + N / hop;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     switch (n_fft) {
-        case 256:  return pg::launch_stft<128>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st);
-        case 512:  return pg::launch_stft<256>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st);
-        case 1024: return pg::launch_stft<512>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st);
-        case 2048: return pg::launch_stft<1024>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st);
+        case 256:  return pg::launch_stft<128>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf);
+        case 512:  return pg::launch_stft<256>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf);
+        case 1024: return pg::launch_stft<512>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf);
+        case 2048: return pg::launch_stft<1024>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf);
     }
     pg::set_error("pg_stft: n_fft must be 256, 512, 1024 or 2048 (got %d)", n_fft);
     return PG_ERR_UNSUPPORTED;
+}
+
+extern "C" int pg_stft(const float* wave, int B, int N, int n_fft, int hop, const float* twiddle, int mode,
+                       float* out_a, float* out_b, uint16_t* op_hi, uint16_t* op_lo,
+                       int64_t op_batch_stride, int op_fmt, pg_stream stream) {
+    return stft_entry(wave, B, N, n_fft, hop, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, nullptr, nullptr, stream);
+}
+
+extern "C" int pg_stft_ragged(const float* wave, int B, int N, int n_fft, int hop, const float* twiddle, int mode,
+                              float* out_a, float* out_b, uint16_t* op_hi, uint16_t* op_lo,
+                              int64_t op_batch_stride, int op_fmt, const int* clip_samples, const int* clip_frames, pg_stream stream) {
+    PG_REQUIRE(clip_samples && clip_frames, "pg_stft_ragged: null per-clip table");
+    if (mode != PG_STFT_LOGMAG) {
+        pg::set_error("pg_stft_ragged: only PG_STFT_LOGMAG takes per-clip lengths (got mode %d)", mode);
+        return PG_ERR_UNSUPPORTED;
+    }
+    return stft_entry(wave, B, N, n_fft, hop, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, clip_samples, clip_frames, stream);
 }
 
 extern "C" int pg_stft_project(const float* wave, int B, int N, int n_fft, int hop, const float* twiddle, const float* mag,
@@ -475,9 +522,9 @@ extern "C" int pg_stft_pairs(const float* wave, int B, int N, int n_fft, int hop
     return PG_ERR_UNSUPPORTED;
 }
 
-extern "C" int pg_istft(const float* in_a, const float* in_b, int mode, int B, int T, int n_fft, int hop,
-                        const float* twiddle, float* wave, float* peak, int* nonfinite,
-                        const float* b_scale_shift, int b_ss_per_clip, pg_stream stream) {
+static int istft_entry(const float* in_a, const float* in_b, int mode, int B, int T, int n_fft, int hop,
+                       const float* twiddle, float* wave, float* peak, int* nonfinite,
+                       const float* b_scale_shift, int b_ss_per_clip, const int* cf, const int* cs, pg_stream stream) {
     PG_REQUIRE(in_a && twiddle && wave && B > 0 && T > 1, "pg_istft: null pointer or empty input");
     PG_REQUIRE(hop * 4 == n_fft, "pg_istft: hop must be n_fft/4 (got n_fft=%d hop=%d)", n_fft, hop);
     PG_REQUIRE(mode >= PG_SPEC_POLAR_LOG && mode <= PG_SPEC_POLAR_MAG, "pg_istft: bad mode %d", mode);
@@ -489,13 +536,27 @@ extern "C" int pg_istft(const float* in_a, const float* in_b, int mode, int B, i
     if (peak) cudaMemsetAsync(peak, 0, sizeof(float) * B, st);
     if (nonfinite) cudaMemsetAsync(nonfinite, 0, sizeof(int) * B, st);
     switch (n_fft) {
-        case 256:  return pg::launch_istft<128>(in_a, in_b, mode, B, T, twiddle, wave, peak, nonfinite, st, b_scale_shift, ss_stride);
-        case 512:  return pg::launch_istft<256>(in_a, in_b, mode, B, T, twiddle, wave, peak, nonfinite, st, b_scale_shift, ss_stride);
-        case 1024: return pg::launch_istft<512>(in_a, in_b, mode, B, T, twiddle, wave, peak, nonfinite, st, b_scale_shift, ss_stride);
-        case 2048: return pg::launch_istft<1024>(in_a, in_b, mode, B, T, twiddle, wave, peak, nonfinite, st, b_scale_shift, ss_stride);
+        case 256:  return pg::launch_istft<128>(in_a, in_b, mode, B, T, twiddle, wave, peak, nonfinite, st, b_scale_shift, ss_stride, cf, cs);
+        case 512:  return pg::launch_istft<256>(in_a, in_b, mode, B, T, twiddle, wave, peak, nonfinite, st, b_scale_shift, ss_stride, cf, cs);
+        case 1024: return pg::launch_istft<512>(in_a, in_b, mode, B, T, twiddle, wave, peak, nonfinite, st, b_scale_shift, ss_stride, cf, cs);
+        case 2048: return pg::launch_istft<1024>(in_a, in_b, mode, B, T, twiddle, wave, peak, nonfinite, st, b_scale_shift, ss_stride, cf, cs);
     }
     pg::set_error("pg_istft: n_fft must be 256, 512, 1024 or 2048 (got %d)", n_fft);
     return PG_ERR_UNSUPPORTED;
+}
+
+extern "C" int pg_istft(const float* in_a, const float* in_b, int mode, int B, int T, int n_fft, int hop,
+                        const float* twiddle, float* wave, float* peak, int* nonfinite,
+                        const float* b_scale_shift, int b_ss_per_clip, pg_stream stream) {
+    return istft_entry(in_a, in_b, mode, B, T, n_fft, hop, twiddle, wave, peak, nonfinite, b_scale_shift, b_ss_per_clip, nullptr, nullptr, stream);
+}
+
+extern "C" int pg_istft_ragged(const float* in_a, const float* in_b, int mode, int B, int T, int n_fft, int hop,
+                               const float* twiddle, float* wave, float* peak, int* nonfinite,
+                               const float* b_scale_shift, int b_ss_per_clip, const int* clip_frames, const int* clip_samples,
+                               pg_stream stream) {
+    PG_REQUIRE(clip_frames && clip_samples, "pg_istft_ragged: null per-clip table");
+    return istft_entry(in_a, in_b, mode, B, T, n_fft, hop, twiddle, wave, peak, nonfinite, b_scale_shift, b_ss_per_clip, clip_frames, clip_samples, stream);
 }
 
 extern "C" int pg_peak_normalize(float* wave, const float* peak, int B, int N, pg_stream stream) {

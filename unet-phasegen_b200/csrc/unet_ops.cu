@@ -108,11 +108,15 @@ __global__ void bn_finalize_kernel(const float4* __restrict__ stats, int B, int 
 // A thread owns a fixed group of four channels -- its (scale, shift) pairs are read once and live in registers (the first
 // version re-read 32 B of them from L1/L2 for every 16 B of payload) -- and walks rows; four rows are loaded before any is
 // stored so that 64 B per thread are in flight.
+// RAGGED: clip b holds valid rows [0, L_b) only (clip_rows[b]); rows [L_b, L) of every destination are written as zeros
+// and y is not read there.
+template <bool RAGGED>
 __global__ void __launch_bounds__(256)
 bn_act_kernel(const float* __restrict__ y, int L, int C, int rows, int ld, const float2* __restrict__ scale_shift,
-              int per_clip, ActDst d0, ActDst d1) {
+              int per_clip, ActDst d0, ActDst d1, const int* __restrict__ clip_rows) {
     const int c4 = C >> 2;
     const int b = blockIdx.y;
+    const int L_b = RAGGED ? min(__ldg(clip_rows + b), L) : L;
     const int tpr = c4 < 256 ? c4 : 256;                    // threads per row (C >= 64 on this path, a multiple of 64)
     const int rpb = 256 / tpr;                              // rows per CTA pass
     const int q0 = threadIdx.x % tpr, r = threadIdx.x / tpr;
@@ -133,7 +137,7 @@ bn_act_kernel(const float* __restrict__ y, int L, int C, int rows, int ld, const
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
                     const int l = l0 + u * step;
-                    if (l < L) v[u] = __ldcs(reinterpret_cast<const float4*>(yb + (size_t)l * ld));   // read once: evict first
+                    if (l < L_b) v[u] = __ldcs(reinterpret_cast<const float4*>(yb + (size_t)l * ld));   // read once: evict first
                 }
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
@@ -142,6 +146,7 @@ bn_act_kernel(const float* __restrict__ y, int L, int C, int rows, int ld, const
                     float4 w = v[u];
                     w.x = fmaf(w.x, s01.x, s01.y); w.y = fmaf(w.y, s01.z, s01.w);
                     w.z = fmaf(w.z, s23.x, s23.y); w.w = fmaf(w.w, s23.z, s23.w);
+                    if (RAGGED && l >= L_b) w = make_float4(0.f, 0.f, 0.f, 0.f);
                     if (d0.dtype) bad0 |= store_act4(d0, b, l, c, w);
                     if (d1.dtype) bad1 |= store_act4(d1, b, l, c, w);
                 }
@@ -280,8 +285,8 @@ extern "C" int pg_bn_finalize(const float* stats, int B, int P, int C, int per_c
     return check_launch("bn_finalize_kernel");
 }
 
-extern "C" int pg_bn_act(const float* y, int B, int L, int C, int rows, int ld, const float* scale_shift, int per_clip,
-                         const pg_act_dst* dst0, const pg_act_dst* dst1, pg_stream stream) {
+static int bn_act_launch(const float* y, int B, int L, int C, int rows, int ld, const float* scale_shift, int per_clip,
+                         const pg_act_dst* dst0, const pg_act_dst* dst1, const int* clip_rows, pg_stream stream) {
     PG_REQUIRE(y && B > 0 && L > 0 && C > 0 && B <= 65535, "pg_bn_act: bad arguments");
     PG_REQUIRE(C % 4 == 0 && ld % 4 == 0, "pg_bn_act: channel count and pitch must be multiples of 4");
     ActDst d0, d1;
@@ -294,9 +299,20 @@ extern "C" int pg_bn_act(const float* y, int B, int L, int C, int rows, int ld, 
     const int want = (148 * 16 + B - 1) / B;
     if (gx > want) gx = want;
     if (gx < 1) gx = 1;
-    bn_act_kernel<<<dim3(gx, B), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
-        y, L, C, rows, ld, reinterpret_cast<const float2*>(scale_shift), per_clip, d0, d1);
+    (clip_rows ? bn_act_kernel<true> : bn_act_kernel<false>)<<<dim3(gx, B), 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+        y, L, C, rows, ld, reinterpret_cast<const float2*>(scale_shift), per_clip, d0, d1, clip_rows);
     return check_launch("bn_act_kernel");
+}
+
+extern "C" int pg_bn_act(const float* y, int B, int L, int C, int rows, int ld, const float* scale_shift, int per_clip,
+                         const pg_act_dst* dst0, const pg_act_dst* dst1, pg_stream stream) {
+    return bn_act_launch(y, B, L, C, rows, ld, scale_shift, per_clip, dst0, dst1, nullptr, stream);
+}
+
+extern "C" int pg_bn_act_ragged(const float* y, int B, int L, int C, int rows, int ld, const float* scale_shift, int per_clip,
+                                const pg_act_dst* dst0, const pg_act_dst* dst1, const int* clip_rows, pg_stream stream) {
+    PG_REQUIRE(clip_rows, "pg_bn_act_ragged: null per-clip row table");
+    return bn_act_launch(y, B, L, C, rows, ld, scale_shift, per_clip, dst0, dst1, clip_rows, stream);
 }
 
 extern "C" int pg_pack_weight(const float* w, int kind, int C_in, int C_out, int k, uint16_t* w_hi, uint16_t* w_lo,

@@ -78,6 +78,10 @@ _SIGNATURES = {
     "pg_unpack_grad": (_I, [_P, _I, _I, _I, _I, _P, _P]),
     "pg_adam_step": (_I, [_P, _P, _I, _P, _P, _L, _F, _F, _F, _F, _I, _F, _P, _P, _P]),
     "pg_cast_split": (_I, [_P, _L, _P, _P, _I, _P, _P]),
+    "pg_stft_ragged": (_I, [_P, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P, _L, _I, _P, _P, _P]),
+    "pg_conv_tc_ragged": (_I, [C.POINTER(ConvDesc), _P, _P, _P, _P, _P, _P, C.POINTER(ConvEpilogue), _P, _P]),
+    "pg_bn_act_ragged": (_I, [_P, _I, _I, _I, _I, _I, _P, _I, C.POINTER(ActDst), C.POINTER(ActDst), _P, _P]),
+    "pg_istft_ragged": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

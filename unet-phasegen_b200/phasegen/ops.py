@@ -65,10 +65,20 @@ def check_stft_geometry(n_fft, hop):
                            f"(got n_fft={n_fft}, hop={hop})")
 
 
-def stft(wave, n_fft, hop, mode=PG_STFT_LOGMAG, want_second=True, operand=None):
+def _lengths(t, B, name):
+    """A per-clip table argument: a contiguous int32 CUDA tensor of B entries."""
+    t = _need_cuda(t, name, torch.int32)
+    if t.numel() != B:
+        raise RuntimeError(f"phasegen: `{name}` must hold one entry per clip ({B}), got {t.numel()}")
+    return t
+
+
+def stft(wave, n_fft, hop, mode=PG_STFT_LOGMAG, want_second=True, operand=None, clip_samples=None, clip_frames=None):
     """wave [B,N] -> (a, b) fp32 [B,T,n_fft/2] frame-major, DC bin dropped.
     mode LOGMAG: a = log1p|X|, b = angle X;  REIM: a = Re X, b = Im X.
-    operand = (hi, lo, batch_stride): also write `a` as bf16 planes (first-conv operand)."""
+    operand = (hi, lo, batch_stride): also write `a` as bf16 planes (first-conv operand).
+    clip_samples / clip_frames (ragged batch, LOGMAG only): int32 CUDA [B], n_b and T_b of each clip (pg_stft_ragged):
+    clip b is its first n_b samples zero-padded to (T_b - 1)*hop, frames >= T_b are 0."""
     check_stft_geometry(n_fft, hop)
     wave = _need_cuda(wave, "wave")
     if wave.dim() != 2:
@@ -79,6 +89,11 @@ def stft(wave, n_fft, hop, mode=PG_STFT_LOGMAG, want_second=True, operand=None):
     a = torch.empty(B, T, Cb, device=wave.device, dtype=torch.float32)
     b = torch.empty_like(a) if want_second else None
     hi, lo, bs = operand if operand is not None else (None, None, 0)
+    if clip_samples is not None or clip_frames is not None:
+        _lib.call("pg_stft_ragged", _ptr(wave), B, N, n_fft, hop, _ptr(twiddle(n_fft, wave.device)), mode,
+                  _ptr(a), _ptr(b), _ptr(hi), _ptr(lo), bs, _fmt(hi), _ptr(_lengths(clip_samples, B, "clip_samples")),
+                  _ptr(_lengths(clip_frames, B, "clip_frames")), _stream())
+        return a, b
     _lib.call("pg_stft", _ptr(wave), B, N, n_fft, hop, _ptr(twiddle(n_fft, wave.device)), mode,
               _ptr(a), _ptr(b), _ptr(hi), _ptr(lo), bs, _fmt(hi), _stream())
     return a, b
@@ -114,11 +129,14 @@ def stft_pairs(wave, n_fft, hop, mean=0.0, std=1.0):
     return lm, ph
 
 
-def istft(a, b, mode, n_fft, hop, normalize=True, check_finite=True, out=None, b_scale_shift=None, bad_out=None):
+def istft(a, b, mode, n_fft, hop, normalize=True, check_finite=True, out=None, b_scale_shift=None, bad_out=None,
+          clip_frames=None, clip_samples=None):
     """(a, b) fp32 [B,T,n_fft/2] frame-major -> wave [B,(T-1)*hop]; optional peak normalisation
     (utils.py:42) and finiteness check (utils.py:41; costs one device->host sync).
     b_scale_shift: float2 per bin, [B, C, 2] (per clip) or [1, C, 2] / [C, 2]: b is read as b*scale + shift (the final
-    norm of the U-Net applied on the fly).  bad_out: int32 [B] buffer that receives the per-clip non-finite flags."""
+    norm of the U-Net applied on the fly).  bad_out: int32 [B] buffer that receives the per-clip non-finite flags.
+    clip_frames / clip_samples (ragged batch): int32 CUDA [B], T_b and n_b of each clip (pg_istft_ragged): clip b is
+    reconstructed from its first T_b frames, its peak and flags cover (T_b - 1)*hop samples, samples >= n_b are 0."""
     check_stft_geometry(n_fft, hop)
     a = _need_cuda(a, "a")
     b = _need_cuda(b, "b") if b is not None else None
@@ -137,8 +155,13 @@ def istft(a, b, mode, n_fft, hop, normalize=True, check_finite=True, out=None, b
         if b_scale_shift.numel() not in (2 * Cb, 2 * Cb * B):
             raise RuntimeError("phasegen.istft: b_scale_shift must hold (scale, shift) per bin, for all clips or per clip")
         per_clip = int(b_scale_shift.numel() == 2 * Cb * B and B > 1)
-    _lib.call("pg_istft", _ptr(a), _ptr(b), mode, B, T, n_fft, hop, _ptr(twiddle(n_fft, a.device)),
-              _ptr(wave), _ptr(peak), _ptr(bad), _ptr(b_scale_shift), per_clip, _stream())
+    if clip_frames is not None or clip_samples is not None:
+        _lib.call("pg_istft_ragged", _ptr(a), _ptr(b), mode, B, T, n_fft, hop, _ptr(twiddle(n_fft, a.device)),
+                  _ptr(wave), _ptr(peak), _ptr(bad), _ptr(b_scale_shift), per_clip,
+                  _ptr(_lengths(clip_frames, B, "clip_frames")), _ptr(_lengths(clip_samples, B, "clip_samples")), _stream())
+    else:
+        _lib.call("pg_istft", _ptr(a), _ptr(b), mode, B, T, n_fft, hop, _ptr(twiddle(n_fft, a.device)),
+                  _ptr(wave), _ptr(peak), _ptr(bad), _ptr(b_scale_shift), per_clip, _stream())
     if normalize:
         _lib.call("pg_peak_normalize", _ptr(wave), _ptr(peak), B, n, _stream())
     if check_finite and bool(bad.any().item()):
@@ -185,9 +208,14 @@ def pack_weight(w, kind, want_tc=True, want_simt=False, plane_dtype=torch.bfloat
     return hi, lo, simt
 
 
-def conv_tc(desc, x_hi, x_lo, w_hi, w_lo, y, stats, epilogue=None):
+def conv_tc(desc, x_hi, x_lo, w_hi, w_lo, y, stats, epilogue=None, out_rows=None):
     """epilogue: a ConvEpilogue (conv_epilogue()) to fuse activation / per-clip norm + activation and the operand-plane
-    writes into the kernel; None = raw fp32 output + statistics records."""
+    writes into the kernel; None = raw fp32 output + statistics records.
+    out_rows (ragged batch): int32 CUDA [B], the valid output rows of each clip (pg_conv_tc_ragged)."""
+    if out_rows is not None:
+        _lib.call("pg_conv_tc_ragged", C.byref(desc), _ptr(x_hi), _ptr(x_lo), _ptr(w_hi), _ptr(w_lo), _ptr(y), _ptr(stats),
+                  C.byref(epilogue) if epilogue is not None else None, _ptr(_lengths(out_rows, desc.B, "out_rows")), _stream())
+        return
     _lib.call("pg_conv_tc", C.byref(desc), _ptr(x_hi), _ptr(x_lo), _ptr(w_hi), _ptr(w_lo), _ptr(y), _ptr(stats),
               C.byref(epilogue) if epilogue is not None else None, _stream())
 
@@ -274,7 +302,12 @@ def bn_from_running(running_mean, running_var, gamma, beta, eps, scale_shift, me
               _ptr(scale_shift), _ptr(mean_var), _stream())
 
 
-def bn_act(y, B, L, Cn, rows, ld, scale_shift, per_clip, dst0, dst1=None):
+def bn_act(y, B, L, Cn, rows, ld, scale_shift, per_clip, dst0, dst1=None, clip_rows=None):
+    """clip_rows (ragged batch): int32 CUDA [B], the valid rows of each clip; rows beyond them are written as 0."""
+    if clip_rows is not None:
+        _lib.call("pg_bn_act_ragged", _ptr(y), B, L, Cn, rows, ld, _ptr(scale_shift), int(per_clip),
+                  C.byref(dst0), C.byref(dst1) if dst1 is not None else None, _ptr(_lengths(clip_rows, B, "clip_rows")), _stream())
+        return
     _lib.call("pg_bn_act", _ptr(y), B, L, Cn, rows, ld, _ptr(scale_shift), int(per_clip),
               C.byref(dst0), C.byref(dst1) if dst1 is not None else None, _stream())
 

@@ -9,6 +9,13 @@ import torch
 
 from . import ops
 from ._lib import PG_DT_F32, PG_PREC_FP32_SIMT, PG_SPEC_POLAR_LOG, PG_STFT_LOGMAG
+from .unet import clip_rows_table, min_frames
+
+
+def ragged_frames(n, hop):
+    """Frames T_b of a clip of n samples in a ragged call: the smallest multiple of 8 with (T_b - 1)*hop >= n (the
+    zero-pad-to-chunk policy of preproc_mdb.py:87-88)."""
+    return (-(-n // hop) + 1 + 7) // 8 * 8
 
 
 class _GraphedPipeline:
@@ -42,25 +49,71 @@ class PhaseGenPipeline:
     def frames(self, n_samples):
         return 1 + n_samples // self.hop
 
-    def __call__(self, wave, check_finite=False, return_intermediates=False, wave_out=None, _precision=None):
+    def ragged_table(self, B, N, lengths, precision=None):
+        """Host int32 table [D+3][B] of a ragged call: row 0 the clip lengths n_b, rows 1 .. D+2 the valid rows of every
+        layer (unet.clip_rows_table of T_b = ragged_frames(n_b)).  Raises ValueError for a call that cannot take them."""
+        levels = self.model._levels()
+        # resolved as in __call__ + model.executor: the call's, the pipeline's, executor_kw's, the model's
+        prec = precision or self.precision or self.executor_kw.get("precision") or self.model._resolve_precision(levels)
+        if prec == "fp32_simt":
+            raise ValueError("lengths: ragged batches run on the tensor-core precisions only, not fp32_simt")
+        if not self.per_clip:
+            raise ValueError("lengths: a ragged batch needs per-clip statistics (per_clip=True); pooled statistics over "
+                             "clips of different lengths have no reference meaning")
+        if isinstance(lengths, torch.Tensor):
+            lengths = lengths.tolist()
+        n = [int(v) for v in lengths]
+        if len(n) != B:
+            raise ValueError(f"lengths holds {len(n)} entries for a batch of {B} clips")
+        T = self.frames(N)
+        if N != (T - 1) * self.hop or T % 8:
+            # the kernels trust T_b <= T (rows of the executor's buffers); that holds for every n_b <= N exactly when
+            # N = (T - 1)*hop with T % 8 == 0, the fixed path's own length rule
+            raise ValueError(f"lengths: the [B, N] buffer must have N = (T - 1)*hop samples with T % 8 == 0 "
+                             f"(got N = {N} at hop {self.hop}); pad it to such a length")
+        if any(v < 0 or v > N for v in n):
+            raise ValueError(f"lengths must lie in [0, {N}] (the samples of the [B, N] buffer), got {n}")
+        T_min = min_frames(levels)
+        T_b = [ragged_frames(v, self.hop) for v in n]
+        if max(T_b) > T:                                    # cannot happen after the check above; the kernels rely on it
+            raise ValueError(f"lengths: a clip needs {max(T_b)} frames, the buffer has {T}")
+        short = [i for i, t in enumerate(T_b) if t < T_min]
+        if short:
+            raise ValueError(f"clips {short} are shorter than the {T_min} frames (at least {(T_min - 9) * self.hop + 1} "
+                             f"samples at hop {self.hop}) the U-Net needs")
+        return [n] + clip_rows_table(levels, T_b)
+
+    def __call__(self, wave, check_finite=False, return_intermediates=False, wave_out=None, lengths=None, _precision=None):
         """wave float32 [B, N] on the GPU, N = (T-1)*hop with T % 8 == 0 -> float32 [B, N].
-        check_finite=True is the finiteness check of utils.py:41 plus the fp16-range guard (one device->host sync)."""
+        check_finite=True is the finiteness check of utils.py:41 plus the fp16-range guard (one device->host sync).
+
+        lengths (a ragged batch): B ints, clip b being wave[b, :n_b].  Its result is the standalone call on that clip
+        zero-padded to (T_b - 1)*hop samples (T_b = ragged_frames(n_b)), peak normalisation included, cut to n_b
+        samples; output samples [n_b, N) are 0 and wave samples >= n_b are never read.  Intermediates hold frames
+        < T_b and zeros beyond.  Needs per_clip=True and a tensor-core precision; the executor is the one of the
+        fixed [B, N] call.  A list of clips becomes such a call through torch.nn.utils.rnn.pad_sequence."""
         if not wave.is_cuda:
             raise RuntimeError("PhaseGenPipeline needs CUDA tensors: there is no CPU fallback")
         B, N = wave.shape
         T = self.frames(N)
         prec = _precision or self.precision
+        table = self.ragged_table(B, N, lengths, prec) if lengths is not None else None
         kw = dict(self.executor_kw)
         if prec:
             kw["precision"] = prec
         ex = self.model.executor(B, T, wave.device, per_clip=self.per_clip, phase_only=self.phase_only, **kw)
         if not any(e is ex for e in self._executors):
             self._executors = (self._executors + [ex])[-8:]
+        rag = {}
+        if table is not None:
+            table = torch.tensor(table, dtype=torch.int32).to(wave.device)   # [n_b; T_b; L_1 .. L_D; T_out]
+            rag = dict(clip_rows=table[1:])
         x0 = ex.x0
         if x0.dtype != PG_DT_F32:
             # the STFT kernel writes the first convolution's 16-bit operand planes directly
             logmag, _ = ops.stft(wave, self.n_fft, self.hop, PG_STFT_LOGMAG, want_second=False,
-                                 operand=(x0.hi, x0.lo, x0.rows * x0.ld))
+                                 operand=(x0.hi, x0.lo, x0.rows * x0.ld),
+                                 **(dict(clip_samples=table[0], clip_frames=table[1]) if rag else {}))
         else:
             logmag, _ = ops.stft(wave, self.n_fft, self.hop, PG_STFT_LOGMAG, want_second=False)
             ex.load_input_cl(logmag)
@@ -69,26 +122,28 @@ class PhaseGenPipeline:
         ss = None
         if ex.C_final == C:
             # the last norm is applied by the ISTFT kernel while it reads the raw phase plane (no normalising pass)
-            phase, ss = self.model._run(ex, dn, up, defer_last=True)
+            phase, ss = self.model._run(ex, dn, up, defer_last=True, **rag)
         else:
-            phase = self.model._run(ex, dn, up)[:, :, :C].contiguous()      # [B, T, 2C] -> phase half
+            phase = self.model._run(ex, dn, up, **rag)[:, :, :C].contiguous()      # [B, T, 2C] -> phase half
         if self._bad is None or self._bad.shape[0] < B or self._bad.device != wave.device:
             self._bad = torch.zeros(max(B, 256), device=wave.device, dtype=torch.int32)
         audio, peak = ops.istft(logmag, phase, PG_SPEC_POLAR_LOG, self.n_fft, self.hop, normalize=self.normalize,
-                                check_finite=False, out=wave_out, b_scale_shift=ss, bad_out=self._bad[:B])
+                                check_finite=False, out=wave_out, b_scale_shift=ss, bad_out=self._bad[:B],
+                                **(dict(clip_frames=table[1], clip_samples=table[0]) if rag else {}))
         if check_finite:
             try:
                 ex.check_range()
             except OverflowError:
                 if self.fp16_overflow == "fallback" and _precision is None:
-                    return self(wave, check_finite, return_intermediates, wave_out, _precision="bf16x3")
+                    return self(wave, check_finite, return_intermediates, wave_out, lengths=lengths, _precision="bf16x3")
                 raise
             if bool(self._bad[:B].any().item()):
                 raise ValueError("Audio buffer is not finite everywhere")
         if return_intermediates:
             if ss is not None:                                  # the normalised phase, materialised for inspection only
                 phase_n = torch.empty_like(phase)
-                ops.bn_act(phase, B, T, C, T, C, ss, self.per_clip, ops.act_dst(phase_n, None, T * C, C, 0, PG_DT_F32, 1.0))
+                ops.bn_act(phase, B, T, C, T, C, ss, self.per_clip, ops.act_dst(phase_n, None, T * C, C, 0, PG_DT_F32, 1.0),
+                           clip_rows=table[-1] if rag else None)
                 phase = phase_n
             return audio, logmag, phase
         return audio

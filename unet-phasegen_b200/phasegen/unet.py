@@ -50,8 +50,44 @@ DEFAULT_BASE_OFFSET_MODE = 0
 
 def _rows(L):
     """Allocated rows per clip: even (the stride-2 parity view reads row L when L is odd) and
-    padded to 8; rows >= L stay zero forever (buffers are zero-initialised, never written)."""
+    padded to 8; rows >= L stay zero forever (buffers are zero-initialised, never written).
+    A ragged call (run(clip_rows=...)) also leaves rows [L_b, L) of clip b zero: every layer writes zeros there."""
     return (L + 7) // 8 * 8
+
+
+def layer_lengths(levels, T):
+    """Rows of every layer of a clip of T frames: [L_0 = T, L_1 .. L_D (down conv outputs), T_out (last up conv
+    output)], or None when the skip concats do not line up (the reference fails in torch.cat there)."""
+    Ld = [T]
+    for lv in levels:
+        Ld.append(lv.down.out_len(Ld[-1]))
+        if Ld[-1] < 1:
+            return None
+    for i in range(len(levels) - 1, 0, -1):
+        if levels[i].up.out_len(Ld[i + 1]) != Ld[i]:
+            return None
+    return Ld + [levels[0].up.out_len(Ld[1])]
+
+
+def min_frames(levels, multiple=8, limit=1 << 16):
+    """Smallest frame count, a multiple of `multiple`, that the U-Net accepts (24 for the reference's)."""
+    for T in range(multiple, limit + 1, multiple):
+        if layer_lengths(levels, T) is not None:
+            return T
+    raise ValueError("phasegen: no frame count up to %d fits this U-Net" % limit)
+
+
+def clip_rows_table(levels, T_list):
+    """Valid-row table of a ragged batch: table[j][b] = layer_lengths(levels, T_list[b])[j], j = 0 .. D+1 (the rows of
+    x0, of the D down-conv outputs and of the last up-conv output).  Raises ValueError for a T the U-Net does not take."""
+    cols = []
+    for T in T_list:
+        L = layer_lengths(levels, int(T))
+        if L is None:
+            raise ValueError(f"phasegen: a clip of {T} frames does not fit this U-Net (minimum {min_frames(levels)}, "
+                             "and the skip connections need T % 8 == 0)")
+        cols.append(L)
+    return [list(r) for r in zip(*cols)]
 
 
 class ConvSpec:
@@ -290,9 +326,12 @@ class UNetExecutor:
             self.wu.append(self._pack_one(up_w[i], lv.up.kind, sl, self.layer_prec("u", i)))
 
     # ------------------------------------------------------------------------------ forward
-    def _conv(self, desc, src, w, y, stats):
+    def _conv(self, desc, src, w, y, stats, rows=None):
         if self.weight_ready is not None:
             self.weight_ready(w)
+        if rows is not None:
+            ops.conv_tc(desc, src.hi, src.lo, w[0], w[1], y, stats, out_rows=rows)
+            return
         if self.prec == PG_PREC_FP32_SIMT:
             ops.conv_simt(desc, src.hi, w[2], y)
             if stats is not None:
@@ -311,20 +350,21 @@ class UNetExecutor:
         else:
             ops.bn_finalize(stats, desc.B, stats.shape[1], desc.C_out, self.per_clip, gamma, beta, eps, ss, mv)
 
-    def _layer(self, mode, desc, src, w, y, stats, ss, mv, norm, running, dst0, dst1=None):
-        """One convolution + (norm) + activation fan-out, in the form chosen at construction."""
+    def _layer(self, mode, desc, src, w, y, stats, ss, mv, norm, running, dst0, dst1=None, rows=None):
+        """One convolution + (norm) + activation fan-out, in the form chosen at construction.  rows: valid output rows
+        per clip (int32 CUDA [B]) of a ragged call."""
         if mode != PG_EPI_RAW:
             if self.weight_ready is not None:
                 self.weight_ready(w)
             gamma, beta, eps = norm if norm is not None else (None, None, BN_EPS_DEFAULT)
             ops.conv_tc(desc, src.hi, src.lo, w[0], w[1], None, None,
-                        ops.conv_epilogue(mode, dst0, dst1, gamma, beta, eps))
+                        ops.conv_epilogue(mode, dst0, dst1, gamma, beta, eps), out_rows=rows)
             return
-        self._conv(desc, src, w, y, stats)
+        self._conv(desc, src, w, y, stats, rows)
         if stats is not None:
             self._finalize(desc, stats, ss, mv, norm, running)
         ops.bn_act(y, desc.B, desc.L_out, desc.C_out, desc.out_rows, desc.out_ld,
-                   ss if stats is not None else None, self.per_clip, dst0, dst1)
+                   ss if stats is not None else None, self.per_clip, dst0, dst1, clip_rows=rows)
 
     def load_input_cf(self, x):
         """x [B,C,T] fp32 (reference layout) -> the level-0 operand (one transposing kernel)."""
@@ -338,28 +378,38 @@ class UNetExecutor:
         B, T, Cn = x_cl.shape
         ops.bn_act(x_cl, B, T, Cn, T, Cn, None, False, self.x0.dst(1.0))
 
-    def run(self, dn_norm, up_norm, defer_last=False, dn_running=None, up_running=None):
+    def run(self, dn_norm, up_norm, defer_last=False, dn_running=None, up_running=None, clip_rows=None):
         """dn_norm/up_norm: per level (gamma, beta, eps) or None.  Consumes self.x0; returns the channels-last
         output [B][T_out][C_final] (a persistent buffer of the executor).  defer_last=True skips the last layer's
         normalising pass and returns (raw output, scale_shift [G][C_final][2]) for a consumer that applies it on the
-        fly (pg_istft).  dn_running/up_running: per level (running_mean, running_var) for use_running executors."""
+        fly (pg_istft).  dn_running/up_running: per level (running_mean, running_var) for use_running executors.
+        clip_rows: ragged batch, int32 CUDA [D+2, B] = clip_rows_table(levels, T_b) with T_b <= T, x0 holding zeros in
+        rows >= T_b.  Every layer then counts rows < L_b of clip b in its statistics and writes zeros into rows
+        [L_b, L) of its destinations, so clip b's valid rows equal a run of that clip alone (per-clip statistics,
+        tensor-core precisions).  The raw output beyond L_b is unspecified."""
         D, lv = self.D, self.levels
+        if clip_rows is not None:
+            if self.prec == PG_PREC_FP32_SIMT or not self.per_clip:
+                raise ValueError("phasegen: ragged batches need per-clip statistics and a tensor-core precision")
+            if tuple(clip_rows.shape) != (D + 2, self.B) or clip_rows.dtype != torch.int32:
+                raise ValueError(f"phasegen: clip_rows must be int32 [{D + 2}, {self.B}]")
+        rows = (lambda j: clip_rows[j]) if clip_rows is not None else (lambda j: None)
         run_of = lambda lst, i: lst[i] if lst is not None else None
         for i in range(D):
             src = self.x0 if i == 0 else self.a[i - 1]
             norm = dn_norm[i] if lv[i].down_norm else None
             dsts = (self.a[i].dst(0.2), self.cat[i].dst(0.0, 0)) if i < D - 1 else (self.a[i].dst(0.0), None)
             self._layer(self.dn_mode[i], self.dn_desc[i], src, self.wd[i], self.z[i], self.dn_stats[i], self.dn_ss[i],
-                        self.dn_mv[i], norm, run_of(dn_running, i), *dsts)
+                        self.dn_mv[i], norm, run_of(dn_running, i), *dsts, rows=rows(i + 1))
         for i in range(D - 1, 0, -1):
             src = self.a[i] if i == D - 1 else self.cat[i]
             norm = up_norm[i] if lv[i].up_norm else None
             self._layer(self.up_mode[i], self.up_desc[i], src, self.wu[i], self.g[i], self.up_stats[i], self.up_ss[i],
-                        self.up_mv[i], norm, run_of(up_running, i), self.cat[i - 1].dst(0.0, lv[i - 1].down.C_out))
+                        self.up_mv[i], norm, run_of(up_running, i), self.cat[i - 1].dst(0.0, lv[i - 1].down.C_out), rows=rows(i))
         # last layer: raw output + statistics, then either the normalising pass or the caller's on-the-fly affine map
         src = self.a[0] if D == 1 else self.cat[0]
         desc, y, stats = self.up_desc[0], self.g[0], self.up_stats[0]
-        self._conv(desc, src, self.wu[0], y, stats)
+        self._conv(desc, src, self.wu[0], y, stats, rows(D + 1))
         norm = up_norm[0] if lv[0].up_norm else None
         if norm is not None and self.C_final != lv[0].up.C_out:
             norm = (norm[0][:self.C_final] if norm[0] is not None else None,
@@ -372,5 +422,6 @@ class UNetExecutor:
         if defer_last and stats is not None:
             return y[:self.B * self.T_out * self.C_final].view(self.B, self.T_out, self.C_final), self.up_ss[0]
         ops.bn_act(y, desc.B, desc.L_out, desc.C_out, desc.out_rows, desc.out_ld, self.up_ss[0] if stats is not None else None,
-                   self.per_clip, ops.act_dst(self.out, None, self.T_out * self.C_final, self.C_final, 0, PG_DT_F32, 1.0))
+                   self.per_clip, ops.act_dst(self.out, None, self.T_out * self.C_final, self.C_final, 0, PG_DT_F32, 1.0),
+                   clip_rows=rows(D + 1))
         return self.out

@@ -91,7 +91,21 @@ int pg_peak_normalize(float* wave, const float* peak, int B, int N, pg_stream st
  * pg_bn_act_ragged: clip_rows[b] = valid rows; y is not read beyond them and rows [L_b, L) of every destination are 0.
  * pg_istft_ragged: frames >= clip_frames[b] are not read; the window sum of squares at the clip's end is the one of
  *   T_b frames; peak and non-finite flags cover samples [0, (T_b - 1)*hop); samples [clip_samples[b], (T-1)*hop) are
- *   written as 0 (pg_peak_normalize keeps them 0). */
+ *   written as 0 (pg_peak_normalize keeps them 0).
+ *
+ * Packed clips: the same clips laid end to end in one flat buffer of n samples, clip b at [o_b, o_b + n_b) with
+ * o_b = clip_offsets[b] (device int64 [B+1], o_0 = 0, o_B = n).  The executor's frame count T is given; the U-Net and ISTFT
+ * entries above run unchanged on [B][T] and [B][(T-1)*hop] buffers.  Offsets are clamped to [0, n] and n_b to >= 0.
+ * pg_stft_packed: pg_stft_ragged of the padded [B][(T-1)*hop] buffer that holds clip b in row b (bit-identical), with the
+ *   clip read from wave[o_b ..] instead; n_b is further clamped to (T-1)*hop.  PG_STFT_LOGMAG only (else PG_ERR_UNSUPPORTED).
+ * pg_peak_normalize_packed: dst[o_b + i] = src[b][i] / peak[b] for i < n_b (src: [B][src_pitch], the pg_istft_ragged output;
+ *   the pg_peak_normalize rule, so bit-identical to it); a copy when peak is NULL.  n_b is clamped to src_pitch, and
+ *   dst [n_dst] is written at [o_b, o_b + n_b) only. */
+int pg_stft_packed(const float* wave, int64_t n_wave, const int64_t* clip_offsets, int B, int T, int n_fft, int hop,
+                   const float* twiddle, int mode, float* out_a, float* out_b, uint16_t* op_hi, uint16_t* op_lo,
+                   int64_t op_batch_stride, int op_fmt, const int* clip_frames, pg_stream stream);
+int pg_peak_normalize_packed(const float* src, int B, int64_t src_pitch, const float* peak, const int64_t* clip_offsets,
+                             float* dst, int64_t n_dst, pg_stream stream);
 int pg_stft_ragged(const float* wave, int B, int N, int n_fft, int hop, const float* twiddle, int mode,
                    float* out_a, float* out_b, uint16_t* op_hi, uint16_t* op_lo, int64_t op_batch_stride,
                    int op_fmt, const int* clip_samples, const int* clip_frames, pg_stream stream);

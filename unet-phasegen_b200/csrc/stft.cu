@@ -63,16 +63,22 @@ __device__ __forceinline__ float fast_log1p_mag(float re, float im) {
 // ------------------------------------------------------------------------------------ STFT
 // FAST = 0: every output selected at run time.  FAST = 1 / 2: the inference path (log-magnitude fp32 plane +
 // bf16 / fp16 hi,lo operand planes, no phase plane) with the selection compiled in.
-// RAGGED: clip b is its first n_b = clip_samples[b] samples zero-padded to N_b = (T_b - 1) * hop, T_b = clip_frames[b]
-// <= T: samples >= n_b are never read, reflect padding happens at N_b, and frames >= T_b are transforms of zeros, so
-// every plane holds exact zeros there.
-template <int NC, int FAST, bool RAGGED>
+// LAYOUT kRagged: clip b is its first n_b = clip_samples[b] samples zero-padded to N_b = (T_b - 1) * hop, T_b =
+// clip_frames[b] <= T: samples >= n_b are never read, reflect padding happens at N_b, and frames >= T_b are transforms of
+// zeros, so every plane holds exact zeros there.
+// LAYOUT kPacked: the same clip program, clip b read from wave[o_b, o_b + n_b) of a flat buffer of n_wave samples,
+// o_b = clip_offsets[b], n_b = clip_offsets[b + 1] - o_b (both clamped to [0, n_wave], n_b to [0, N]).  Whether a clip
+// takes the float2 loads depends on its own offset; an interior frame of an odd-offset clip takes two unchecked scalar
+// loads instead, so only edge frames pay for the reflect and bounds checks.
+enum { kFixed = 0, kRagged = 1, kPacked = 2 };
+template <int NC, int FAST, int LAYOUT>
 __global__ void __launch_bounds__(kStftThreads, 3)          // 3 CTAs per SM (<= 85 registers): the kernel is issue/latency-bound
 stft_kernel(const float* __restrict__ wave, int N, int T, const float2* __restrict__ tw_g, int mode,
             float* __restrict__ out_a, float* __restrict__ out_b,
             uint16_t* __restrict__ op_hi, uint16_t* __restrict__ op_lo,
             long long op_batch_stride, int op_fmt, int frames_per_cta, const float* __restrict__ proj_mag,
-            float std_mean, float std_inv, const int* __restrict__ clip_samples, const int* __restrict__ clip_frames) {
+            float std_mean, float std_inv, const int* __restrict__ clip_samples, const int* __restrict__ clip_frames,
+            const long long* __restrict__ clip_offsets, long long n_wave) {
     using Cfg = FrameCfg<NC>;
     using R = Radix<NC, false>;
     extern __shared__ float2 smem2[];
@@ -87,28 +93,45 @@ stft_kernel(const float* __restrict__ wave, int N, int T, const float2* __restri
         win[m] = {0.25f - 0.25f * tw_g[2 * m].x, 0.25f - 0.25f * tw_g[2 * m + 1].x};   // post-processing folded in
     __syncthreads();
 
+    constexpr bool RAGGED = LAYOUT != kFixed;               // per-clip frame counts (ragged and packed)
     const int b = blockIdx.y;
-    const int n_b = RAGGED ? min(__ldg(clip_samples + b), N) : N;   // samples read from the clip
+    // packed: the clip's offset o_b is re-read from shared memory at every frame; held in registers across the frame
+    // program it pushes the n_fft 2048 / 1024 variants past the 80 registers of 3 CTAs per SM
+    __shared__ long long clip_base;
+    int n_b = N;
+    if (LAYOUT == kPacked) {
+        const long long o_b = min(max(__ldg(clip_offsets + b), 0ll), n_wave);
+        const long long e_b = min(max(__ldg(clip_offsets + b + 1), o_b), n_wave);
+        n_b = (int)min(e_b - o_b, (long long)N);            // samples read from the clip
+        if (tid == 0) clip_base = o_b;
+        __syncthreads();
+    } else if (LAYOUT == kRagged) {
+        n_b = min(__ldg(clip_samples + b), N);
+    }
     const int T_b = RAGGED ? min(__ldg(clip_frames + b), T) : T;
     const int N_b = RAGGED ? (T_b - 1) * Cfg::HOP : N;      // where the reflect padding happens
     const int slot = tid / Cfg::TG, t = tid % Cfg::TG;
     cpx* s = bufs + slot * Cfg::PL;
     const FrameSync<Cfg::TG> sync{slot};
-    const float* w = wave + (size_t)b * N;
-    const bool aligned = (N & 1) == 0 && (reinterpret_cast<uintptr_t>(wave) & 7) == 0;   // float2 loads
+    const float* w_row = wave + (size_t)b * N;
+    const bool aligned_row = (N & 1) == 0 && (reinterpret_cast<uintptr_t>(wave) & 7) == 0;   // float2 loads
     const int f_begin = blockIdx.x * frames_per_cta;
 
     for (int f0 = f_begin; f0 < f_begin + frames_per_cta && f0 < T; f0 += Cfg::FC) {
+        const float* w = LAYOUT == kPacked ? wave + clip_base : w_row;
+        const bool aligned = LAYOUT == kPacked ? (reinterpret_cast<uintptr_t>(w) & 7) == 0 : aligned_row;   // per clip
         const int frame = f0 + slot;
         const bool live = frame < T;
         // padded sample p <-> wave index p - n_fft/2, reflected at both ends (librosa center=True)
         const int p0 = frame * Cfg::HOP - NC;
         cpx v[16];
-        if (live && aligned && p0 >= 0 && p0 + Cfg::NFFT <= n_b) {
+        if (live && (LAYOUT == kPacked || aligned) && p0 >= 0 && p0 + Cfg::NFFT <= n_b) {
 #pragma unroll
             for (int r = 0; r < 16; ++r) {
                 const int m = t + r * Cfg::TG;
-                const float2 xv = __ldg(reinterpret_cast<const float2*>(w + p0) + m);
+                float2 xv;
+                if (LAYOUT != kPacked || aligned) xv = __ldg(reinterpret_cast<const float2*>(w + p0) + m);
+                else xv = make_float2(__ldg(w + p0 + 2 * m), __ldg(w + p0 + 2 * m + 1));   // interior frame, odd clip offset
                 const cpx wv = win[m];
                 v[r] = {xv.x * wv.x, xv.y * wv.y};
             }
@@ -354,6 +377,48 @@ __global__ void peak_normalize_kernel(float* __restrict__ wave, const unsigned* 
     }
 }
 
+// Packs the ISTFT's padded plane: dst[o_b + i] = src[b][i] / peak_b for i < n_b (the librosa.util.normalize rule of
+// peak_normalize_kernel, so the result is bit-identical to normalising in place and slicing), a plain copy when
+// peak_bits is NULL or the peak is tiny.  Offsets are clamped to [0, n_dst] and n_b to [0, src_pitch], so a bad table
+// writes inside dst and reads inside row b only.  float4 stores once dst is 16-byte aligned, float4 loads too when
+// src sits at the same alignment; else scalar loads.
+__global__ void __launch_bounds__(256)
+peak_normalize_packed_kernel(const float* __restrict__ src, long long src_pitch, const unsigned* __restrict__ peak_bits,
+                             const long long* __restrict__ clip_offsets, float* __restrict__ dst, long long n_dst) {
+    const int b = blockIdx.y;
+    const long long o = min(max(__ldg(clip_offsets + b), 0ll), n_dst);
+    const long long e = min(max(__ldg(clip_offsets + b + 1), o), n_dst);
+    const long long n = min(e - o, src_pitch);
+    const float pk = peak_bits ? __uint_as_float(__ldg(peak_bits + b)) : 0.f;
+    const bool scale = pk >= 1.17549435e-38f;
+    const float inv = scale ? 1.0f / pk : 1.0f;
+    const float* s = src + (size_t)b * src_pitch;
+    float* d = dst + o;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    const long long i0 = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    // head: scalar up to the first 16-byte aligned dst address
+    const long long head = min((long long)((16 - (reinterpret_cast<uintptr_t>(d) & 15)) & 15) / 4, n);
+    for (long long i = i0; i < head; i += stride) d[i] = scale ? s[i] * inv : s[i];
+    const long long n4 = (n - head) / 4;
+    float4* d4 = reinterpret_cast<float4*>(d + head);
+    const float* sh = s + head;
+    if ((reinterpret_cast<uintptr_t>(sh) & 15) == 0) {
+        const float4* s4 = reinterpret_cast<const float4*>(sh);
+        for (long long i = i0; i < n4; i += stride) {
+            float4 v = __ldg(s4 + i);
+            if (scale) { v.x *= inv; v.y *= inv; v.z *= inv; v.w *= inv; }
+            d4[i] = v;
+        }
+    } else {
+        for (long long i = i0; i < n4; i += stride) {
+            float4 v = make_float4(__ldg(sh + 4 * i), __ldg(sh + 4 * i + 1), __ldg(sh + 4 * i + 2), __ldg(sh + 4 * i + 3));
+            if (scale) { v.x *= inv; v.y *= inv; v.z *= inv; v.w *= inv; }
+            d4[i] = v;
+        }
+    }
+    for (long long i = head + 4 * n4 + i0; i < n; i += stride) d[i] = scale ? s[i] * inv : s[i];
+}
+
 // Long-form stitching (BASELINE.json config 4): windows of `win` samples every `step` samples (step >= win/2, so at
 // most two overlap) are cross-faded with a periodic-Hann ramp over the ov = win - step shared samples (rising half on
 // the later window, falling half on the earlier one: the two gains sum to one).  Window i sits at slot
@@ -390,32 +455,35 @@ stitch_kernel(const float* __restrict__ windows, int n_windows, int win, int ste
     }
 }
 
-template <int NC, bool RAGGED>
+template <int NC, int LAYOUT>
 static auto stft_variant(bool fast, int fmt) {
-    return !fast ? stft_kernel<NC, 0, RAGGED> : fmt == PG_FMT_F16 ? stft_kernel<NC, 2, RAGGED> : stft_kernel<NC, 1, RAGGED>;
+    return !fast ? stft_kernel<NC, 0, LAYOUT> : fmt == PG_FMT_F16 ? stft_kernel<NC, 2, LAYOUT> : stft_kernel<NC, 1, LAYOUT>;
 }
 
 template <int NC>
 static int launch_stft(const float* wave, int B, int N, int T, const float* tw, int mode, float* a, float* bq,
                        uint16_t* hi, uint16_t* lo, long long bs, int fmt, cudaStream_t st, const float* proj_mag = nullptr,
-                       float std_mean = 0.f, float std_inv = 1.f, const int* clip_samples = nullptr, const int* clip_frames = nullptr) {
+                       float std_mean = 0.f, float std_inv = 1.f, const int* clip_samples = nullptr, const int* clip_frames = nullptr,
+                       const long long* clip_offsets = nullptr, long long n_wave = 0) {
     using Cfg = FrameCfg<NC>;
     const bool fast = mode == PG_STFT_LOGMAG && a && !bq && hi && lo;
-    auto k = clip_samples ? stft_variant<NC, true>(fast, fmt) : stft_variant<NC, false>(fast, fmt);
+    auto k = clip_offsets ? stft_variant<NC, kPacked>(fast, fmt)
+           : clip_samples ? stft_variant<NC, kRagged>(fast, fmt) : stft_variant<NC, kFixed>(fast, fmt);
     const size_t sm = Cfg::smem_stft();
     static bool configured_dev[kMaxDevices] = {};
     bool& configured = configured_dev[current_device_slot()];
     if (!configured) {
         for (int f = 0; f < 3; ++f)
-            for (auto kv : {stft_variant<NC, false>(f > 0, f == 2 ? PG_FMT_F16 : PG_FMT_BF16),
-                            stft_variant<NC, true>(f > 0, f == 2 ? PG_FMT_F16 : PG_FMT_BF16)})
+            for (auto kv : {stft_variant<NC, kFixed>(f > 0, f == 2 ? PG_FMT_F16 : PG_FMT_BF16),
+                            stft_variant<NC, kRagged>(f > 0, f == 2 ? PG_FMT_F16 : PG_FMT_BF16),
+                            stft_variant<NC, kPacked>(f > 0, f == 2 ? PG_FMT_F16 : PG_FMT_BF16)})
                 cudaFuncSetAttribute(kv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
         configured = true;
     }
     const int frames_per_cta = Cfg::FC * 4;                 // tables are built once per 4 passes over the frame slots
     dim3 grid((T + frames_per_cta - 1) / frames_per_cta, B);
     k<<<grid, kStftThreads, sm, st>>>(wave, N, T, reinterpret_cast<const float2*>(tw), mode, a, bq, hi, lo, bs, fmt, frames_per_cta, proj_mag,
-                                      std_mean, std_inv, clip_samples, clip_frames);
+                                      std_mean, std_inv, clip_samples, clip_frames, clip_offsets, n_wave);
     return check_launch("stft_kernel");
 }
 
@@ -450,7 +518,8 @@ extern "C" int pg_stft_num_frames(int n_samples, int hop) { return hop > 0 ? 1 +
 
 static int stft_entry(const float* wave, int B, int N, int n_fft, int hop, const float* twiddle, int mode,
                       float* out_a, float* out_b, uint16_t* op_hi, uint16_t* op_lo,
-                      int64_t op_batch_stride, int op_fmt, const int* cs, const int* cf, pg_stream stream) {
+                      int64_t op_batch_stride, int op_fmt, const int* cs, const int* cf, pg_stream stream,
+                      const int64_t* co = nullptr, int64_t n_wave = 0) {
     PG_REQUIRE(wave && twiddle && B > 0 && N > 0, "pg_stft: null pointer or empty batch");
     PG_REQUIRE(hop * 4 == n_fft, "pg_stft: hop must be n_fft/4 (got n_fft=%d hop=%d)", n_fft, hop);
     PG_REQUIRE(N > n_fft / 2, "pg_stft: reflect padding needs more than n_fft/2 samples (N=%d)", N);
@@ -459,10 +528,14 @@ static int stft_entry(const float* wave, int B, int N, int n_fft, int hop, const
     const int T = 1 + N / hop;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     switch (n_fft) {
-        case 256:  return pg::launch_stft<128>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf);
-        case 512:  return pg::launch_stft<256>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf);
-        case 1024: return pg::launch_stft<512>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf);
-        case 2048: return pg::launch_stft<1024>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf);
+        case 256:  return pg::launch_stft<128>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf,
+                                                 reinterpret_cast<const long long*>(co), n_wave);
+        case 512:  return pg::launch_stft<256>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf,
+                                                 reinterpret_cast<const long long*>(co), n_wave);
+        case 1024: return pg::launch_stft<512>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf,
+                                                 reinterpret_cast<const long long*>(co), n_wave);
+        case 2048: return pg::launch_stft<1024>(wave, B, N, T, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, st, nullptr, 0.f, 1.f, cs, cf,
+                                                 reinterpret_cast<const long long*>(co), n_wave);
     }
     pg::set_error("pg_stft: n_fft must be 256, 512, 1024 or 2048 (got %d)", n_fft);
     return PG_ERR_UNSUPPORTED;
@@ -483,6 +556,19 @@ extern "C" int pg_stft_ragged(const float* wave, int B, int N, int n_fft, int ho
         return PG_ERR_UNSUPPORTED;
     }
     return stft_entry(wave, B, N, n_fft, hop, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt, clip_samples, clip_frames, stream);
+}
+
+extern "C" int pg_stft_packed(const float* wave, int64_t n_wave, const int64_t* clip_offsets, int B, int T, int n_fft, int hop,
+                              const float* twiddle, int mode, float* out_a, float* out_b, uint16_t* op_hi, uint16_t* op_lo,
+                              int64_t op_batch_stride, int op_fmt, const int* clip_frames, pg_stream stream) {
+    PG_REQUIRE(clip_offsets && clip_frames && n_wave > 0, "pg_stft_packed: null per-clip table or empty buffer");
+    PG_REQUIRE(T >= 2 && hop > 0 && (int64_t)(T - 1) * hop <= INT32_MAX, "pg_stft_packed: bad frame count T=%d", T);
+    if (mode != PG_STFT_LOGMAG) {
+        pg::set_error("pg_stft_packed: only PG_STFT_LOGMAG takes packed clips (got mode %d)", mode);
+        return PG_ERR_UNSUPPORTED;
+    }
+    return stft_entry(wave, B, (T - 1) * hop, n_fft, hop, twiddle, mode, out_a, out_b, op_hi, op_lo, op_batch_stride, op_fmt,
+                      nullptr, clip_frames, stream, clip_offsets, n_wave);
 }
 
 extern "C" int pg_stft_project(const float* wave, int B, int N, int n_fft, int hop, const float* twiddle, const float* mag,
@@ -565,6 +651,17 @@ extern "C" int pg_peak_normalize(float* wave, const float* peak, int B, int N, p
     pg::peak_normalize_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
         wave, reinterpret_cast<const unsigned*>(peak), N);
     return pg::check_launch("peak_normalize_kernel");
+}
+
+extern "C" int pg_peak_normalize_packed(const float* src, int B, int64_t src_pitch, const float* peak,
+                                        const int64_t* clip_offsets, float* dst, int64_t n_dst, pg_stream stream) {
+    PG_REQUIRE(src && clip_offsets && dst && B > 0 && B <= 65535 && src_pitch > 0 && n_dst >= 0,
+               "pg_peak_normalize_packed: bad arguments");
+    const int64_t per = (src_pitch + 1023) / 1024;
+    dim3 grid(per < 64 ? (unsigned)per : 64u, B);
+    pg::peak_normalize_packed_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(
+        src, src_pitch, reinterpret_cast<const unsigned*>(peak), reinterpret_cast<const long long*>(clip_offsets), dst, n_dst);
+    return pg::check_launch("peak_normalize_packed_kernel");
 }
 
 extern "C" int pg_stitch(const float* windows, int n_windows, int win, int step, int world, int per_rank, float* out,

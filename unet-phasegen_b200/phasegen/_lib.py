@@ -82,6 +82,8 @@ _SIGNATURES = {
     "pg_conv_tc_ragged": (_I, [C.POINTER(ConvDesc), _P, _P, _P, _P, _P, _P, C.POINTER(ConvEpilogue), _P, _P]),
     "pg_bn_act_ragged": (_I, [_P, _I, _I, _I, _I, _I, _P, _I, C.POINTER(ActDst), C.POINTER(ActDst), _P, _P]),
     "pg_istft_ragged": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P, _I, _P, _P, _P]),
+    "pg_stft_packed": (_I, [_P, _L, _P, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P, _L, _I, _P, _P]),
+    "pg_peak_normalize_packed": (_I, [_P, _I, _L, _P, _P, _P, _L, _P]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

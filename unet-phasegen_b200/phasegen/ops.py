@@ -65,22 +65,36 @@ def check_stft_geometry(n_fft, hop):
                            f"(got n_fft={n_fft}, hop={hop})")
 
 
-def _lengths(t, B, name):
-    """A per-clip table argument: a contiguous int32 CUDA tensor of B entries."""
-    t = _need_cuda(t, name, torch.int32)
+def _lengths(t, B, name, dtype=torch.int32):
+    """A per-clip table argument: a contiguous int32 (int64 for offsets) CUDA tensor of B entries."""
+    t = _need_cuda(t, name, dtype)
     if t.numel() != B:
         raise RuntimeError(f"phasegen: `{name}` must hold one entry per clip ({B}), got {t.numel()}")
     return t
 
 
-def stft(wave, n_fft, hop, mode=PG_STFT_LOGMAG, want_second=True, operand=None, clip_samples=None, clip_frames=None):
+def stft(wave, n_fft, hop, mode=PG_STFT_LOGMAG, want_second=True, operand=None, clip_samples=None, clip_frames=None,
+         clip_offsets=None, frames=None):
     """wave [B,N] -> (a, b) fp32 [B,T,n_fft/2] frame-major, DC bin dropped.
     mode LOGMAG: a = log1p|X|, b = angle X;  REIM: a = Re X, b = Im X.
     operand = (hi, lo, batch_stride): also write `a` as bf16 planes (first-conv operand).
     clip_samples / clip_frames (ragged batch, LOGMAG only): int32 CUDA [B], n_b and T_b of each clip (pg_stft_ragged):
-    clip b is its first n_b samples zero-padded to (T_b - 1)*hop, frames >= T_b are 0."""
+    clip b is its first n_b samples zero-padded to (T_b - 1)*hop, frames >= T_b are 0.
+    clip_offsets (packed clips, LOGMAG only, with clip_frames and `frames` = T): int64 CUDA [B+1]; wave is 1-D and clip b
+    is wave[o_b:o_(b+1)], otherwise as the ragged batch (pg_stft_packed)."""
     check_stft_geometry(n_fft, hop)
     wave = _need_cuda(wave, "wave")
+    if clip_offsets is not None:
+        if wave.dim() != 1 or frames is None or clip_frames is None:
+            raise RuntimeError("phasegen.stft: packed clips need a 1-D wave, clip_frames and frames")
+        B, T, Cb = clip_offsets.numel() - 1, int(frames), n_fft // 2
+        a = torch.empty(B, T, Cb, device=wave.device, dtype=torch.float32)
+        b = torch.empty_like(a) if want_second else None
+        hi, lo, bs = operand if operand is not None else (None, None, 0)
+        _lib.call("pg_stft_packed", _ptr(wave), wave.numel(), _ptr(_lengths(clip_offsets, B + 1, "clip_offsets", torch.int64)),
+                  B, T, n_fft, hop, _ptr(twiddle(n_fft, wave.device)), mode, _ptr(a), _ptr(b), _ptr(hi), _ptr(lo), bs,
+                  _fmt(hi), _ptr(_lengths(clip_frames, B, "clip_frames")), _stream())
+        return a, b
     if wave.dim() != 2:
         raise RuntimeError("phasegen.stft: wave must be [B, N]")
     B, N = wave.shape
@@ -167,6 +181,23 @@ def istft(a, b, mode, n_fft, hop, normalize=True, check_finite=True, out=None, b
     if check_finite and bool(bad.any().item()):
         raise ValueError("Audio buffer is not finite everywhere")
     return wave, peak
+
+
+def peak_normalize_packed(src, peak, clip_offsets, out):
+    """Pack the rows of src [B, n] (an ISTFT output) into out [sum n_b] (pg_peak_normalize_packed):
+    out[o_b + i] = src[b, i] / peak[b] for i < n_b = o_(b+1) - o_b, the pg_peak_normalize rule; a copy when peak is None.
+    clip_offsets: int64 CUDA [B+1]."""
+    src = _need_cuda(src, "src")
+    if src.dim() != 2:
+        raise RuntimeError("phasegen.peak_normalize_packed: src must be [B, n]")
+    B = src.shape[0]
+    peak = _lengths(peak, B, "peak", torch.float32) if peak is not None else None
+    offs = _lengths(clip_offsets, B + 1, "clip_offsets", torch.int64)
+    if not (isinstance(out, torch.Tensor) and out.dim() == 1 and out.is_contiguous()):
+        raise RuntimeError("phasegen.peak_normalize_packed: `out` must be a contiguous 1-D CUDA float32 tensor")
+    _need_cuda(out, "out")
+    _lib.call("pg_peak_normalize_packed", _ptr(src), B, src.shape[1], _ptr(peak), _ptr(offs), _ptr(out), out.numel(), _stream())
+    return out
 
 
 def transpose(src, dst=None, dst_hi=None, dst_lo=None, dst_batch_stride=None, dst_ld=None, range_flag=None):

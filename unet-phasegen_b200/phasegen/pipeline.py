@@ -5,6 +5,8 @@ preproc_mdb.py:93 (STFT), data.py:39-47 (log-magnitude), demo.py:33-42 (per-clip
 forward, polar->complex, generate_audio) for a whole batch of clips, without the
 numpy/CPU round trips the reference makes at demo.py:37-40.
 """
+import itertools
+
 import torch
 
 from . import ops
@@ -16,6 +18,34 @@ def ragged_frames(n, hop):
     """Frames T_b of a clip of n samples in a ragged call: the smallest multiple of 8 with (T_b - 1)*hop >= n (the
     zero-pad-to-chunk policy of preproc_mdb.py:87-88)."""
     return (-(-n // hop) + 1 + 7) // 8 * 8
+
+
+def packed_offsets(lengths):
+    """Offsets o_0 .. o_B of clips laid end to end: clip b is flat[o_b:o_(b+1)]."""
+    return [0] + list(itertools.accumulate(int(v) for v in lengths))
+
+
+def chunk_sizes(B, chunks, name="run_host"):
+    """Sub-batch sizes of a host call: `chunks` equal ones (the last may be shorter), or an explicit list adding up to B."""
+    if isinstance(chunks, int):
+        per = -(-B // max(1, chunks))
+        return [min(per, B - c0) for c0 in range(0, B, per)]
+    sizes = [int(c) for c in chunks]
+    if sum(sizes) != B or min(sizes) < 1:
+        raise RuntimeError(f"{name}: chunk sizes {sizes} do not add up to the batch of {B}")
+    return sizes
+
+
+def packed_sub_batches(lengths, chunks):
+    """Sub-batches of a packed batch for run_host_packed: per sub-batch (c0, c1, s0, s1, offsets) with clips [c0, c1),
+    samples [s0, s1) of the flat buffer (one contiguous copy each way) and the offsets of its clips rebased to s0."""
+    offs = packed_offsets(lengths)
+    out, c0 = [], 0
+    for n in chunk_sizes(len(offs) - 1, chunks, "run_host_packed"):
+        c1 = c0 + n
+        out.append((c0, c1, offs[c0], offs[c1], [o - offs[c0] for o in offs[c0:c1 + 1]]))
+        c0 = c1
+    return out
 
 
 class _GraphedPipeline:
@@ -45,6 +75,8 @@ class PhaseGenPipeline:
         self.executor_kw = dict(executor_kw or {})     # extra UNetExecutor options (e.g. fuse=False: the two-pass norm form)
         self._executors = []
         self._bad = None
+        self._planes = {}                              # packed calls' padded ISTFT planes, per (B, T, device)
+        self._host_states = {}                         # run_host / run_host_packed streams and staging buffers
 
     def frames(self, n_samples):
         return 1 + n_samples // self.hop
@@ -83,6 +115,26 @@ class PhaseGenPipeline:
                              f"samples at hop {self.hop}) the U-Net needs")
         return [n] + clip_rows_table(levels, T_b)
 
+    def packed_table(self, flat, lengths, frames=None, precision=None):
+        """Host tables of a packed call: (T, table, offsets).  T is the executor's frame count (`frames`, by default
+        ragged_frames(max n_b)), table the ragged_table of the padded [B, (T - 1)*hop] call and offsets the B + 1 clip
+        offsets in `flat`.  Raises ValueError for a call that cannot take them."""
+        if flat.dim() != 1:
+            raise ValueError(f"packed clips: the flat buffer must be 1-D, got shape {tuple(flat.shape)}")
+        if isinstance(lengths, torch.Tensor):
+            lengths = lengths.tolist()
+        n = [int(v) for v in lengths]
+        if not n:
+            raise ValueError("packed clips: lengths is empty")
+        if sum(n) != flat.numel():
+            raise ValueError(f"packed clips: the lengths add up to {sum(n)} samples, the flat buffer holds {flat.numel()}")
+        T_max = ragged_frames(max(n), self.hop)
+        T = T_max if frames is None else int(frames)
+        if T % 8 or T < T_max:
+            raise ValueError(f"packed clips: frames must be a multiple of 8 and at least {T_max} (the longest clip's "
+                             f"frame count), got {frames}")
+        return T, self.ragged_table(len(n), (T - 1) * self.hop, n, precision), packed_offsets(n)
+
     def __call__(self, wave, check_finite=False, return_intermediates=False, wave_out=None, lengths=None, _precision=None):
         """wave float32 [B, N] on the GPU, N = (T-1)*hop with T % 8 == 0 -> float32 [B, N].
         check_finite=True is the finiteness check of utils.py:41 plus the fp16-range guard (one device->host sync).
@@ -91,33 +143,61 @@ class PhaseGenPipeline:
         zero-padded to (T_b - 1)*hop samples (T_b = ragged_frames(n_b)), peak normalisation included, cut to n_b
         samples; output samples [n_b, N) are 0 and wave samples >= n_b are never read.  Intermediates hold frames
         < T_b and zeros beyond.  Needs per_clip=True and a tensor-core precision; the executor is the one of the
-        fixed [B, N] call.  A list of clips becomes such a call through torch.nn.utils.rnn.pad_sequence."""
+        fixed [B, N] call.  A list of clips becomes such a call through torch.nn.utils.rnn.pad_sequence, or without
+        padding through `packed`."""
         if not wave.is_cuda:
             raise RuntimeError("PhaseGenPipeline needs CUDA tensors: there is no CPU fallback")
         B, N = wave.shape
-        T = self.frames(N)
         prec = _precision or self.precision
-        table = self.ragged_table(B, N, lengths, prec) if lengths is not None else None
+        table = None
+        if lengths is not None:                             # [n_b; T_b; L_1 .. L_D; T_out]
+            table = torch.tensor(self.ragged_table(B, N, lengths, prec), dtype=torch.int32).to(wave.device)
+        return self._forward(wave, B, self.frames(N), table, None, prec, check_finite, return_intermediates, wave_out,
+                             _precision is None)
+
+    def packed(self, flat, lengths, frames=None, check_finite=False, return_intermediates=False, out=None):
+        """Packed clips: flat float32 1-D on the GPU holding B clips end to end (clip b = flat[o_b:o_b + n_b],
+        o_b = n_0 + .. + n_(b-1), lengths = [n_0 .. n_(B-1)], sum n_b == flat.numel()) -> float32 1-D of the same
+        layout.  Clip b's result, and its intermediates ([B, T, C] as in the ragged call), are bit-identical to the
+        ragged call pipe(padded, lengths=lengths) on the [B, (T - 1)*hop] buffer holding clip b in row b: same
+        executor, tables and kernels; only the STFT reads and the final peak-normalise pass writes the packed layout.
+        frames: the executor's frame count T, by default ragged_frames(max n_b); a larger multiple of 8 keeps one
+        executor for a range of batches.  out: a contiguous CUDA float32 1-D tensor of flat.numel() elements."""
+        T, table, offsets = self.packed_table(flat, lengths, frames, self.precision)
+        if not flat.is_cuda:
+            raise RuntimeError("PhaseGenPipeline needs CUDA tensors: there is no CPU fallback")
+        if out is not None and (not out.is_cuda or out.dtype != torch.float32 or out.dim() != 1 or not out.is_contiguous()
+                                or out.numel() != flat.numel()):
+            raise RuntimeError(f"packed: `out` must be a contiguous CUDA float32 1-D tensor of {flat.numel()} elements")
+        table = torch.tensor(table, dtype=torch.int32).to(flat.device)
+        offsets = torch.tensor(offsets, dtype=torch.int64).to(flat.device)
+        return self._forward(flat, len(offsets) - 1, T, table, offsets, self.precision, check_finite, return_intermediates,
+                             out, True)
+
+    def _forward(self, src, B, T, table, offsets, prec, check_finite, return_intermediates, out, may_fall_back):
+        """The body of a call: src [B, (T-1)*hop] (fixed or ragged: table = None or the device int32 ragged_table) or
+        a packed 1-D buffer (offsets = device int64 [B+1]; its ISTFT writes a per-(B, T) scratch plane that the
+        peak-normalise pass packs into `out`)."""
         kw = dict(self.executor_kw)
         if prec:
             kw["precision"] = prec
-        ex = self.model.executor(B, T, wave.device, per_clip=self.per_clip, phase_only=self.phase_only, **kw)
+        ex = self.model.executor(B, T, src.device, per_clip=self.per_clip, phase_only=self.phase_only, **kw)
         if not any(e is ex for e in self._executors):
             self._executors = (self._executors + [ex])[-8:]
-        rag = {}
-        if table is not None:
-            table = torch.tensor(table, dtype=torch.int32).to(wave.device)   # [n_b; T_b; L_1 .. L_D; T_out]
-            rag = dict(clip_rows=table[1:])
+        rag = dict(clip_rows=table[1:]) if table is not None else {}
         x0 = ex.x0
         if x0.dtype != PG_DT_F32:
             # the STFT kernel writes the first convolution's 16-bit operand planes directly
-            logmag, _ = ops.stft(wave, self.n_fft, self.hop, PG_STFT_LOGMAG, want_second=False,
-                                 operand=(x0.hi, x0.lo, x0.rows * x0.ld),
-                                 **(dict(clip_samples=table[0], clip_frames=table[1]) if rag else {}))
+            if offsets is not None:
+                clips = dict(clip_frames=table[1], clip_offsets=offsets, frames=T)
+            else:
+                clips = dict(clip_samples=table[0], clip_frames=table[1]) if rag else {}
+            logmag, _ = ops.stft(src, self.n_fft, self.hop, PG_STFT_LOGMAG, want_second=False,
+                                 operand=(x0.hi, x0.lo, x0.rows * x0.ld), **clips)
         else:
-            logmag, _ = ops.stft(wave, self.n_fft, self.hop, PG_STFT_LOGMAG, want_second=False)
+            logmag, _ = ops.stft(src, self.n_fft, self.hop, PG_STFT_LOGMAG, want_second=False)
             ex.load_input_cl(logmag)
-        dn, up = self.model._norm_params(wave.device)
+        dn, up = self.model._norm_params(src.device)
         C = self.n_fft // 2
         ss = None
         if ex.C_final == C:
@@ -125,17 +205,23 @@ class PhaseGenPipeline:
             phase, ss = self.model._run(ex, dn, up, defer_last=True, **rag)
         else:
             phase = self.model._run(ex, dn, up, **rag)[:, :, :C].contiguous()      # [B, T, 2C] -> phase half
-        if self._bad is None or self._bad.shape[0] < B or self._bad.device != wave.device:
-            self._bad = torch.zeros(max(B, 256), device=wave.device, dtype=torch.int32)
-        audio, peak = ops.istft(logmag, phase, PG_SPEC_POLAR_LOG, self.n_fft, self.hop, normalize=self.normalize,
-                                check_finite=False, out=wave_out, b_scale_shift=ss, bad_out=self._bad[:B],
+        if self._bad is None or self._bad.shape[0] < B or self._bad.device != src.device:
+            self._bad = torch.zeros(max(B, 256), device=src.device, dtype=torch.int32)
+        packed = offsets is not None
+        audio, peak = ops.istft(logmag, phase, PG_SPEC_POLAR_LOG, self.n_fft, self.hop, normalize=self.normalize and not packed,
+                                check_finite=False, out=self._packed_plane(B, T, src.device) if packed else out,
+                                b_scale_shift=ss, bad_out=self._bad[:B],
                                 **(dict(clip_frames=table[1], clip_samples=table[0]) if rag else {}))
+        if packed:
+            # the normalise pass packs the padded plane (a copy when normalize=False): no extra pass over the audio
+            audio = ops.peak_normalize_packed(audio, peak if self.normalize else None, offsets,
+                                              out if out is not None else torch.empty(src.numel(), device=src.device))
         if check_finite:
             try:
                 ex.check_range()
             except OverflowError:
-                if self.fp16_overflow == "fallback" and _precision is None:
-                    return self(wave, check_finite, return_intermediates, wave_out, lengths=lengths, _precision="bf16x3")
+                if self.fp16_overflow == "fallback" and may_fall_back:
+                    return self._forward(src, B, T, table, offsets, "bf16x3", check_finite, return_intermediates, out, False)
                 raise
             if bool(self._bad[:B].any().item()):
                 raise ValueError("Audio buffer is not finite everywhere")
@@ -147,6 +233,16 @@ class PhaseGenPipeline:
                 phase = phase_n
             return audio, logmag, phase
         return audio
+
+    def _packed_plane(self, B, T, device):
+        """The padded [B, (T - 1)*hop] ISTFT output of packed calls: scratch, one per (B, T, device)."""
+        planes = self._planes
+        key = (B, T, device)
+        if key not in planes:
+            if len(planes) >= 8:
+                planes.clear()
+            planes[key] = torch.empty(B, (T - 1) * self.hop, device=device)
+        return planes[key]
 
     def range_overflow(self):
         """Sticky fp16-range flags of every executor this pipeline has used, read and cleared (one small device->host
@@ -235,64 +331,134 @@ class PhaseGenPipeline:
         if host_in.is_cuda or host_out.is_cuda:
             raise RuntimeError("run_host takes host tensors; call the pipeline directly for device tensors")
         B, N = host_in.shape
-        if isinstance(chunks, int):
-            per = -(-B // max(1, chunks))
-            sizes = [min(per, B - c0) for c0 in range(0, B, per)]
-        else:
-            sizes = [int(c) for c in chunks]
-            if sum(sizes) != B or min(sizes) < 1:
-                raise RuntimeError(f"run_host: chunk sizes {sizes} do not add up to the batch of {B}")
+        sizes = chunk_sizes(B, chunks)
+        starts = list(itertools.accumulate([0] + sizes))
+        dev = torch.cuda.current_stream().device
+        e_out = self._host_loop(
+            ("rows", tuple(sizes), N, dev), sizes, pipelined,
+            stage=lambda n: (torch.empty(n, N, device=dev), torch.empty(n, N, device=dev)),
+            upload=lambda k, d_in: d_in.copy_(host_in[starts[k]:starts[k + 1]], non_blocking=True),
+            compute=lambda k, d_in, d_out, tab: self(d_in, wave_out=d_out),
+            download=lambda k, d_out: host_out[starts[k]:starts[k + 1]].copy_(d_out, non_blocking=True))
+        return e_out if pipelined else host_out
+
+    def run_host_packed(self, host_in, lengths, host_out, chunks=4, frames=None, pipelined=False):
+        """`packed` on HOST buffers: pinned float32 1-D in and out, clips end to end as in `packed`, with the contract
+        of run_host (sub-batches whose copies overlap the GPU work; pipelined=True returns the event of the last
+        download).  Sub-batch k holds clips [c0, c0 + n) and copies samples [o_c0, o_(c0+n)) in and out, one
+        contiguous copy each way, so no padding crosses PCIe.  Every sub-batch runs at the same frame count T
+        (`frames`, by default that of the longest clip of the batch); its staging buffers hold n*(T - 1)*hop samples
+        and are allocated once per (sub-batch sizes, T, device), so a stream of batches with different lengths and
+        the same `frames` reuses them.  The per-clip tables of all sub-batches are uploaded in one copy from a pinned
+        buffer before the first sub-batch's samples.  suggest_chunks(B, (T - 1)*hop, device[, stream=True]) gives
+        sub-batch sizes that fill whole waves of the convolution grid.  Each clip's result is bit-identical to
+        `packed` on its sub-batch with the same `frames`."""
+        if host_in.is_cuda or host_out.is_cuda:
+            raise RuntimeError("run_host_packed takes host tensors; call `packed` for device tensors")
+        T, table, _ = self.packed_table(host_in, lengths, frames, self.precision)
+        if host_out.dim() != 1 or host_out.numel() != host_in.numel():
+            raise RuntimeError(f"run_host_packed: host_out must be 1-D with {host_in.numel()} elements")
+        subs = packed_sub_batches(table[0], chunks)
+        sizes = [c1 - c0 for c0, c1, _, _, _ in subs]
+        R = len(table)
+        # one host buffer for every sub-batch's tables: the int64 rebased offsets of all sub-batches, then their int32
+        # [R, n] ragged tables (every part a multiple of 8 bytes long when it is int64, so each view stays aligned)
+        parts = [torch.tensor(o, dtype=torch.int64).view(torch.uint8) for _, _, _, _, o in subs]
+        parts += [torch.tensor([row[c0:c1] for row in table], dtype=torch.int32).view(-1).view(torch.uint8)
+                  for c0, c1, _, _, _ in subs]
+        at = list(itertools.accumulate([0] + [p.numel() for p in parts]))
+        tables = torch.cat(parts)
+        K = len(subs)
+        span = (T - 1) * self.hop
+        dev = torch.cuda.current_stream().device
+
+        def compute(k, d_in, d_out, tab):
+            c0, c1, s0, s1, _ = subs[k]
+            offs = tab[at[k]:at[k + 1]].view(torch.int64)
+            rows = tab[at[K + k]:at[K + k + 1]].view(torch.int32).view(R, c1 - c0)
+            self._forward(d_in[:s1 - s0], c1 - c0, T, rows, offs, self.precision, False, False, d_out[:s1 - s0], False)
+
+        e_out = self._host_loop(
+            ("packed", tuple(sizes), T, dev, tables.numel()), sizes, pipelined,
+            stage=lambda n: (torch.empty(n * span, device=dev), torch.empty(n * span, device=dev)),
+            upload=lambda k, d_in: d_in[:subs[k][3] - subs[k][2]].copy_(host_in[subs[k][2]:subs[k][3]], non_blocking=True),
+            compute=compute,
+            download=lambda k, d_out: host_out[subs[k][2]:subs[k][3]].copy_(d_out[:subs[k][3] - subs[k][2]], non_blocking=True),
+            tables=tables)
+        return e_out if pipelined else host_out
+
+    def _host_loop(self, key, sizes, pipelined, stage, upload, compute, download, tables=None):
+        """The stream / event / staging loop of run_host and run_host_packed.  key[0] names the form; a new key
+        replaces that form's streams and buffers.  stage(n) -> (d_in, d_out), the device staging buffers of a sub-batch
+        of n clips (allocated once per key and staging set); upload(k, d_in) and download(k, d_out) enqueue the copies
+        of sub-batch k (on the upload / download stream), compute(k, d_in, d_out, tab) its GPU work (on the current
+        stream).  tables (CPU uint8, the same size for every call of a key): copied into the set's pinned buffer and
+        uploaded in one copy ahead of the first sub-batch; compute receives the device copy.  Returns the event of the
+        last download (pipelined) or None after ordering the downloads on the current stream."""
         cur = torch.cuda.current_stream()
         dev = cur.device
-        st = getattr(self, "_host_state", None)
-        key = (tuple(sizes), N, dev)
+        st = self._host_states.get(key[0])
         if st is None or st["key"] != key:
             if st is not None:                              # a new batch geometry: let the old staging buffers drain before they are freed
                 st["s_in"].synchronize()
                 st["s_out"].synchronize()
             st = {"key": key, "s_in": torch.cuda.Stream(device=dev), "s_out": torch.cuda.Stream(device=dev), "sets": [], "calls": 0}
-            self._host_state = st
+            self._host_states[key[0]] = st
         # the stream-of-batches form alternates between two sets of staging buffers, so the uploads of batch i+1 never
         # wait for batch i's GPU work (with one sub-batch per batch that is the whole difference between copy + compute
         # and max(copy, compute)); the one-batch-at-a-time form uses the first set only
         which = st["calls"] & 1 if pipelined else 0
         st["calls"] += 1 if pipelined else 0
         while len(st["sets"]) <= which:
-            st["sets"].append({"d_in": [torch.empty(n, N, device=dev) for n in sizes], "d_out": [torch.empty(n, N, device=dev) for n in sizes],
-                               "consumed": [None] * len(sizes), "drained": [None] * len(sizes)})
+            bufs = [stage(n) for n in sizes]
+            st["sets"].append({"d_in": [b[0] for b in bufs], "d_out": [b[1] for b in bufs],
+                               "consumed": [None] * len(sizes), "drained": [None] * len(sizes),
+                               "tab_host": None, "tab_dev": None, "tab_sent": None})
         s_in, s_out, st = st["s_in"], st["s_out"], st["sets"][which]
         if not pipelined:
             s_in.wait_stream(cur)
             s_out.wait_stream(cur)
-        c0 = 0
+        tab = None
+        if tables is not None:
+            if st["tab_host"] is None:
+                st["tab_host"] = torch.empty_like(tables).pin_memory()
+                st["tab_dev"] = torch.empty_like(tables, device=dev)
+            elif st["tab_sent"] is not None:
+                st["tab_sent"].synchronize()                # the last upload from the pinned buffer has read it
+            st["tab_host"].copy_(tables)
+            if st["consumed"][-1] is not None:
+                s_in.wait_event(st["consumed"][-1])         # the previous batch on this set has run (and read the tables)
+            with torch.cuda.stream(s_in):
+                st["tab_dev"].copy_(st["tab_host"], non_blocking=True)
+                st["tab_sent"] = torch.cuda.Event()
+                st["tab_sent"].record(s_in)
+            tab = st["tab_dev"]
         e_out = None
-        for k, n in enumerate(sizes):
-            sl = slice(c0, c0 + n)
-            c0 += n
+        for k in range(len(sizes)):
             d_in, d_out = st["d_in"][k], st["d_out"][k]
             if st["consumed"][k] is not None:
                 s_in.wait_event(st["consumed"][k])          # the previous batch's sub-batch k has been read by its STFT
             with torch.cuda.stream(s_in):
-                d_in.copy_(host_in[sl], non_blocking=True)
+                upload(k, d_in)
                 e_in = torch.cuda.Event()
                 e_in.record(s_in)
             cur.wait_event(e_in)
             if st["drained"][k] is not None:
                 cur.wait_event(st["drained"][k])            # the previous batch's output k has been downloaded
-            self(d_in, wave_out=d_out)
+            compute(k, d_in, d_out, tab)
             e_done = torch.cuda.Event()
             e_done.record(cur)
             st["consumed"][k] = e_done
             s_out.wait_event(e_done)
             with torch.cuda.stream(s_out):
-                host_out[sl].copy_(d_out, non_blocking=True)
+                download(k, d_out)
                 e_out = torch.cuda.Event()
                 e_out.record(s_out)
             st["drained"][k] = e_out
         if pipelined:
             return e_out                                    # s_out is in order: the last download's event covers them all
         cur.wait_stream(s_out)
-        return host_out
+        return None
 
 
 def ramp_sizes(B, cap, nb, max_waves=6):

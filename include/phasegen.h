@@ -83,8 +83,9 @@ int pg_peak_normalize(float* wave, const float* peak, int B, int N, pg_stream st
  * [L_b, L), which is the zero padding the next convolution of the standalone clip would read.  Table entries larger
  * than the call's extent (N, T, L_out, L) are clamped to it, so a bad table never reaches another clip's rows.
  *
- * pg_stft_ragged: PG_STFT_LOGMAG only (else PG_ERR_UNSUPPORTED).  Samples >= clip_samples[b] are never read; reflect
- *   padding at (T_b - 1)*hop; frames >= T_b = clip_frames[b] are written as 0 in every plane.
+ * pg_stft_ragged: PG_STFT_LOGMAG only (else PG_ERR_UNSUPPORTED).  Clip b is its first min(clip_samples[b], (T_b - 1)*hop)
+ *   samples: later samples are never read, even when clip_samples[b] is larger; reflect padding at (T_b - 1)*hop;
+ *   frames >= T_b = clip_frames[b] are written as 0 in every plane.  The result does not depend on the buffer's alignment.
  * pg_conv_tc_ragged: out_rows[b] = valid output rows L_b.  PG_EPI_RAW: statistics records count those rows only (a part
  *   with none gets n = 0, which pg_bn_finalize skips); y beyond them is unspecified.  PG_EPI_ACT / NORM_ACT: the norm
  *   uses those rows only and rows [L_b, L_out) of both destinations are written as 0.
@@ -97,7 +98,8 @@ int pg_peak_normalize(float* wave, const float* peak, int B, int N, pg_stream st
  * o_b = clip_offsets[b] (device int64 [B+1], o_0 = 0, o_B = n).  The executor's frame count T is given; the U-Net and ISTFT
  * entries above run unchanged on [B][T] and [B][(T-1)*hop] buffers.  Offsets are clamped to [0, n] and n_b to >= 0.
  * pg_stft_packed: pg_stft_ragged of the padded [B][(T-1)*hop] buffer that holds clip b in row b (bit-identical), with the
- *   clip read from wave[o_b ..] instead; n_b is further clamped to (T-1)*hop.  PG_STFT_LOGMAG only (else PG_ERR_UNSUPPORTED).
+ *   clip read from wave[o_b ..] instead; n_b is further clamped to (T_b - 1)*hop, T_b = clip_frames[b], so samples of the
+ *   next clip are never read, whatever the offset's alignment.  PG_STFT_LOGMAG only (else PG_ERR_UNSUPPORTED).
  * pg_peak_normalize_packed: dst[o_b + i] = src[b][i] / peak[b] for i < n_b (src: [B][src_pitch], the pg_istft_ragged output;
  *   the pg_peak_normalize rule, so bit-identical to it); a copy when peak is NULL.  n_b is clamped to src_pitch, and
  *   dst [n_dst] is written at [o_b, o_b + n_b) only. */

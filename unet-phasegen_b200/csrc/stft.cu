@@ -63,11 +63,12 @@ __device__ __forceinline__ float fast_log1p_mag(float re, float im) {
 // ------------------------------------------------------------------------------------ STFT
 // FAST = 0: every output selected at run time.  FAST = 1 / 2: the inference path (log-magnitude fp32 plane +
 // bf16 / fp16 hi,lo operand planes, no phase plane) with the selection compiled in.
-// LAYOUT kRagged: clip b is its first n_b = clip_samples[b] samples zero-padded to N_b = (T_b - 1) * hop, T_b =
+// LAYOUT kRagged: clip b is its first n_b = min(clip_samples[b], N_b) samples zero-padded to N_b = (T_b - 1) * hop, T_b =
 // clip_frames[b] <= T: samples >= n_b are never read, reflect padding happens at N_b, and frames >= T_b are transforms of
-// zeros, so every plane holds exact zeros there.
+// zeros, so every plane holds exact zeros there.  A table with n_b > N_b thus gives the same result on every buffer
+// alignment (the float2 path is gated by n_b alone).
 // LAYOUT kPacked: the same clip program, clip b read from wave[o_b, o_b + n_b) of a flat buffer of n_wave samples,
-// o_b = clip_offsets[b], n_b = clip_offsets[b + 1] - o_b (both clamped to [0, n_wave], n_b to [0, N]).  Whether a clip
+// o_b = clip_offsets[b], n_b = clip_offsets[b + 1] - o_b (both clamped to [0, n_wave], n_b to [0, N_b]).  Whether a clip
 // takes the float2 loads depends on its own offset; an interior frame of an odd-offset clip takes two unchecked scalar
 // loads instead, so only edge frames pay for the reflect and bounds checks.
 enum { kFixed = 0, kRagged = 1, kPacked = 2 };
@@ -110,6 +111,7 @@ stft_kernel(const float* __restrict__ wave, int N, int T, const float2* __restri
     }
     const int T_b = RAGGED ? min(__ldg(clip_frames + b), T) : T;
     const int N_b = RAGGED ? (T_b - 1) * Cfg::HOP : N;      // where the reflect padding happens
+    if (RAGGED) n_b = min(n_b, N_b);                        // samples past the clip's padded end are never read
     const int slot = tid / Cfg::TG, t = tid % Cfg::TG;
     cpx* s = bufs + slot * Cfg::PL;
     const FrameSync<Cfg::TG> sync{slot};
